@@ -2,6 +2,7 @@
 """bench.py — env-steps/s of the Craft hot path (teacher action + features + step) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--envs-per-gpu E] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 One "step" = one rollout tick of the whole batch: for every env the BFS teacher's action, the
 f32[404] feature vector and the state transition (with done / success / auto-reset), i.e. the body
@@ -30,6 +31,7 @@ UNIT = "env-steps/s"
 # algorithmic bytes per env-step at craft_medium (SURVEY.md §8(d), DESIGN.md §"Rooflines")
 BYTES_FUSED = 1815
 BYTES_STEP, BYTES_FEATURES, BYTES_EXPERT = 198, 1712, 97
+DUMP_BYTES = 60 * 10**6          # --dump-outputs: all arrays together, with room for the .npy headers
 
 
 def load_workload(n_envs, split="train"):
@@ -241,6 +243,20 @@ def oracle_parity_sample(env, tables, wl_arrays, snap, out, feat_ring, ticks, fi
             "against": "oracle/craft_oracle.c, advanced tick by tick from the pre-launch state"}
 
 
+def last_step_outputs(torch, features, out, row, n):
+    """What one step hands its caller — the f32 feature frame, the teacher's actions and the done /
+    success flags — as float arrays on the device.  Larger batches are cut to a fixed, seeded sample of
+    envs (``env_index``) so that all arrays together stay under DUMP_BYTES."""
+    per_env = 4 * features.shape[-1] + 4 * 3 + 8
+    m = min(n, DUMP_BYTES // per_env)
+    envs = np.arange(n) if m == n else np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+    idx = torch.from_numpy(envs).to(features.device)
+    res = {"env_index": torch.from_numpy(envs.astype(np.float64)), "features": features[idx]}
+    for k in ("expert", "done", "success"):
+        res[k] = (out[k] if row is None else out[k][row])[idx].float()
+    return res
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -382,43 +398,35 @@ def run_ours(args):
     prepare(ring * 8)
 
     sampler = ClockSampler(local) if rank == 0 else None
-    run_steps(max(W, 3))
     run_steps(K)                                    # one untimed pass of the K-step plan: graph upload
-    torch.cuda.synchronize()
-    # ---- how many times the K-step plan is repeated so that the timed region lasts >= 50 ms
-    s0, s1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    s0.record()
-    run_steps(K)
-    s1.record()
-    torch.cuda.synchronize()
-    est = torch.tensor([s0.elapsed_time(s1) * 1e-3], dtype=torch.float64, device=dev)
-    if distributed:
-        dist.all_reduce(est, op=dist.ReduceOp.MIN)          # same R on every rank
-    R = int(min(4000, max(1, np.ceil(args.min_seconds / max(float(est.item()), 1e-7)))))
-    if args.repeats > 0:
-        R = args.repeats
+    # where the last of K steps leaves its outputs: the plan's last launch runs K % T (or T) ticks and
+    # writes the frame of tick t to ring slot t; one tick per launch: step j writes slot j % ring
+    tl = K % T or T
+    last_step = ((feat_ring[tl - 1], routs[tl], tl - 1) if T > 1 else
+                 (feats[(K - 1) % ring], outs[(K - 1) % ring], None))
     env.stats.zero_()
     ticks_before = ticks_done[0]
     phase0 = (40 - env.timer.to(torch.int64)).cpu().numpy()      # ticks into the running episode, per env
     torch.cuda.synchronize()
     if distributed:
         dist.barrier()
-    marks = [torch.cuda.Event(enable_timing=True) for _ in range(R + 1)]
-    torch.cuda.synchronize()
+    m0, m1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t0 = time.time()
+    # the warm-up is still running when the first event is queued, so the timed region starts with
+    # the K-step plan already submitted instead of measuring its submission
+    run_steps(max(W, 3))
     launches[0] = 0
-    marks[0].record()
-    for r in range(R):                              # exactly K steps per repeat, events in between
-        run_steps(K)
-        marks[r + 1].record()
+    m0.record()
+    run_steps(K)                                    # the timed region: exactly K steps
+    m1.record()
     timed_launches = launches[0]
     torch.cuda.synchronize()
     t1 = time.time()
     if distributed:
         dist.barrier()
-    per_rep = torch.tensor([marks[r].elapsed_time(marks[r + 1]) * 1e-3 for r in range(R)],
-                           dtype=torch.float64, device=dev)
-    total = torch.tensor([marks[0].elapsed_time(marks[R]) * 1e-3], dtype=torch.float64, device=dev)
+    # what the last timed step returned, sampled before anything else runs on the envs
+    dumped = last_step_outputs(torch, *last_step, n) if args.dump_outputs and rank == 0 else None
+    total = torch.tensor([m0.elapsed_time(m1) * 1e-3], dtype=torch.float64, device=dev)
     stats = env.stats.clone()
     # Size-independent invariant over the WHOLE timed region (every launch, chained or not): teacher-
     # driven episodes of instance i last exactly ref_len[i] ticks and always succeed, so the number of
@@ -431,8 +439,8 @@ def run_ours(args):
         local = stats.cpu().numpy()
         episodes_ok = bool(int(local[0]) == expected and int(local[1]) == expected)
         assert episodes_ok, "episodes %d / successes %d, expected %d" % (local[0], local[1], expected)
+    counted_steps = n * world * (ticks_done[0] - ticks_before)
     if distributed:
-        dist.all_reduce(per_rep, op=dist.ReduceOp.MAX)      # MAX over ranks, repeat by repeat
         dist.all_reduce(total, op=dist.ReduceOp.MAX)
     ar0, ar1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ar0.record()
@@ -440,8 +448,7 @@ def run_ours(args):
     ar1.record()
     torch.cuda.synchronize()
     stats_allreduce_us = ar0.elapsed_time(ar1) * 1e3
-    elapsed = float(per_rep.median().item())                # seconds per K steps (median of R)
-    total_s = float(total.item())
+    elapsed = float(total.item())                           # seconds for the K timed steps, MAX over ranks
     clocks = None
     if sampler:
         t1c, window = t1, "timed region"
@@ -456,10 +463,14 @@ def run_ours(args):
         clocks = sampler.stop(t0, t1c)
         clocks["window"] = window
     env.check_errors()
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a.cpu().numpy())
     total_steps = n * K * world
     value = total_steps / elapsed
     st = stats.cpu().numpy()
-    assert int(st[2]) == total_steps * R, "kernel step counter disagrees with the host's"
+    assert int(st[2]) == counted_steps, "kernel step counter disagrees with the host's"
 
     # ---- parity of the timed kernel: one more replay of the SAME K-step plan, the last launch of
     # it checked against the CPU oracle on a strided sample (untimed)
@@ -515,7 +526,7 @@ def run_ours(args):
     per_tick_s = elapsed / K             # seconds per tick (= per step)
     line = {
         "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,
-        "repeats": R, "timed_region_ms": total_s * 1e3,
+        "timed_region_ms": elapsed * 1e3,
         "ms_per_step": per_tick_s * 1e3, "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": "u8", "data": "synthetic",
         "config": {
@@ -525,16 +536,15 @@ def run_ours(args):
             "kernel": ("craft_rollout_kernel (fused tick, %d ticks per launch)" % T if T > 1 else
                        "craft_tick_kernel (fused, warp-specialised)") if fused else "expert+features+advance",
             "cuda_graph": graph is not None,
-            "timing": "the K-step plan is replayed `repeats` times back to back with CUDA events in "
-                      "between (one untimed replay first); value = envs x K / median per-K time, MAX over "
-                      "ranks per repeat; timed_region_ms is the whole window",
+            "timing": "one untimed replay of the K-step plan, then the warm-up and the K timed steps "
+                      "queued back to back, CUDA events around the K steps; value = envs x K / their time, "
+                      "MAX over ranks",
             "l2": "feature outputs rotate through a ring of %d frames (%.0f MB > 126 MB L2); tick t of a "
                   "launch writes slot t %% ring, so a line is rewritten only after >= 850 MB of other "
                   "writes" % (ring, ring * feat_bytes / 1e6),
         },
         "clocks": clocks,
-        "gpu_launches": timed_launches // R,
-        "gpu_launches_timed_region": timed_launches,
+        "gpu_launches": timed_launches,
         "parity_checked": parity is not None, "parity": parity,
         "episodes_match_closed_form": episodes_ok,
         "stats_allreduce_us": stats_allreduce_us if distributed else None,
@@ -555,8 +565,8 @@ def run_ours(args):
     if fused:
         # per env: T x (404 f32 features + action + done + success) + one state read and write
         bytes_per_tick = BYTES_FUSED if T == 1 else (1616 + 3) + (2 * 96 + 4) / T
-        launch_s = elapsed * R / max(1, timed_launches)
-        ticks_per_launch_eff = K * R / max(1, timed_launches)
+        launch_s = elapsed / max(1, timed_launches)
+        ticks_per_launch_eff = K / max(1, timed_launches)
         achieved = bytes_per_tick * ticks_per_launch_eff * n / launch_s / 1e9
         line["roofline"] = {"bound": "hbm", "kernel": "craft_rollout_kernel" if T > 1 else "craft_tick_kernel",
                             "achieved": achieved, "peak": peak, "unit": "GB/s", "frac": achieved / peak,
@@ -1073,9 +1083,9 @@ def main():
                     help="chunk size of the u8-on-the-wire e2e form (profiles/bench_runs/r2_e2e_wire_sweep.txt)")
     ap.add_argument("--ticks-per-launch", type=int, default=8,
                     help="teacher-driven rollouts run this many ticks per kernel launch (1 = one tick per launch)")
-    ap.add_argument("--min-seconds", type=float, default=0.06,
-                    help="the K-step plan is repeated until the timed region lasts at least this long")
-    ap.add_argument("--repeats", type=int, default=0, help="force the number of repeats (0 = from --min-seconds)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned on rank 0 (features, teacher actions, done / "
+                         "success flags; a fixed sample of envs beyond %d MB) as DIR/<name>.npy" % (DUMP_BYTES // 10**6))
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle check of the timed kernel")
     ap.add_argument("--no-1m", action="store_true", help="skip the 1,048,576-env per-kernel table")
     ap.add_argument("--no-config3", action="store_true", help="skip BASELINE config 3 (world > 1)")

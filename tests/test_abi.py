@@ -82,19 +82,6 @@ def test_tables_match_reference_ids(medium_tables):
     assert medium_tables.task_len[24] == 14
 
 
-def test_tables_from_reference_yaml_if_present(medium_tables):
-    ref = "/root/reference/resources/craft"
-    if not os.path.isdir(ref):
-        pytest.skip("reference checkout not present")
-    from psketch_b200.tables import Cookbook, CraftTables, TaskManager
-    t2 = CraftTables(Cookbook(os.path.join(ref, "recipes.yaml")),
-                     TaskManager(os.path.join(ref, "hints.hierarchy.yaml")))
-    assert np.array_equal(t2.kind_class, medium_tables.kind_class)
-    assert np.array_equal(t2.recipes, medium_tables.recipes)
-    assert np.array_equal(t2.task_nodes, medium_tables.task_nodes)
-    assert np.array_equal(t2.task_len, medium_tables.task_len)
-
-
 def test_rollout_kernel_register_budget(lib_path):
     """The multi-tick kernel is built for 896 threads per SM: 7 CTAs of 64 env threads + 2 feature
     warps, or 9 CTAs of 32 + 2 (the shape used from 65,536 envs up: 2,048 CTAs on 1,332 slots).

@@ -33,17 +33,22 @@ def test_wire_format_accepts_both_task_spellings(medium_tables):
 
 
 def test_dataset_mirror_batches_like_the_reference(splits, medium_tables, tmp_path):
-    """Dataset (data/dataset.py:12-93): same flattening and the same shuffled batch order for the
-    same RandomState; compared with the reference class itself when the checkout is present."""
+    """Dataset (data/dataset.py:12-93): same flattening, and the same shuffled batch order as the
+    reference's own Dataset — the 30 training batches its ImitationTrainer drew with RandomState(123),
+    as recorded in tests/golden/config4_imitation.npz."""
     import json
     import os
-    import sys
     import types
     from psketch_b200 import data
-    packed = {k[4:]: splits[k] for k in splits.files if k.startswith("dev_")}
-    packed["inst_env"] = packed["inst_env"].astype(np.int32)
-    packed["ref_len"] = packed["ref_len"].astype(np.int32)
-    json.dump(data.to_wire(packed, medium_tables), open(str(tmp_path / "craft_medium_dev.json"), "w"))
+
+    def write(split):
+        packed = {k[len(split) + 1:]: splits[k] for k in splits.files if k.startswith(split + "_")}
+        packed["inst_env"] = packed["inst_env"].astype(np.int32)
+        packed["ref_len"] = packed["ref_len"].astype(np.int32)
+        json.dump(data.to_wire(packed, medium_tables), open(str(tmp_path / ("craft_medium_%s.json" % split)), "w"))
+        return packed
+    packed = write("dev")
+    write("train")
 
     def cfg(seed):
         return types.SimpleNamespace(data_dir=str(tmp_path), world=types.SimpleNamespace(config="craft_medium"),
@@ -56,22 +61,13 @@ def test_dataset_mirror_batches_like_the_reference(splits, medium_tables, tmp_pa
     assert len(batches) == 69 and len(batches[-1]) == 2200 - 68 * 32
     back = ds.packed(medium_tables)
     assert np.array_equal(back["inst_pos"], packed["inst_pos"]) and np.array_equal(back["ref_actions"], packed["ref_actions"])
-    ref_root = "/root/reference"
-    if not os.path.isdir(os.path.join(ref_root, "data")):
-        return
-    sys.path.insert(0, ref_root)
-    try:
-        import importlib
-        for m in [m for m in sys.modules if m == "data" or m.startswith("data.")]:
-            del sys.modules[m]
-        ref_ds_mod = importlib.import_module("data.dataset")
-    finally:
-        sys.path.remove(ref_root)
-    rds = ref_ds_mod.Dataset(cfg(3), "dev", medium_tables.task_manager)
-    rb = list(rds.iterate_batches())
-    assert [[it["id"] for it in b] for b in rb] == [[it["id"] for it in b] for b in batches]
-    assert all(a["init_pos"] == b["init_pos"] and a["ref_actions"] == b["ref_actions"]
-               for a, b in zip(rds.data, ds.data))
+    rec = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "config4_imitation.npz"))
+    train = data.Dataset(cfg(123), "train", medium_tables.task_manager)
+    row = {it["id"]: i for i, it in enumerate(train.data)}
+    batches = train.iterate_batches()
+    for r in range(int(rec["n_train_iters"])):
+        got = [row[it["id"]] for it in next(batches)]
+        assert got == rec["batch"][r, :int(rec["n_env"][r])].tolist(), r
 
 
 def test_traj_files_have_the_reference_format(tmp_path):

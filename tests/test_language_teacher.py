@@ -1,8 +1,7 @@
-"""Language teachers (host word logic): same outputs and same random-stream consumption as the
-reference's teachers/primitive_language.py when that checkout is present, fixed expectations
-otherwise.  CPU only (fake states: ``describe`` reads just .pos and .inventory)."""
-import os
-import sys
+"""Language teachers (host word logic): fixed expectations, and the batched forms against the
+per-rollout ones.  Same words, learned action map and random-stream use as the reference's
+teachers/primitive_language.py are pinned by the record of the reference's own training run
+(tests/test_config4.py).  CPU only (fake states: ``describe`` reads just .pos and .inventory)."""
 import types
 
 import numpy as np
@@ -53,23 +52,8 @@ def test_instruct_and_describe():
     assert ids.tolist() == [[2, 5, 6, 0]]
     eps = _episodes(np.random.RandomState(1))
     mine = [t.describe(world, a, s) for a, s in eps]
-    ref_root = "/root/reference"
-    if not os.path.isdir(os.path.join(ref_root, "teachers")):
-        assert all(len(m) == len(a) for m, (a, _) in zip(mine, eps))
-        assert len(t.student_action_map) >= 4
-        return
-    sys.path.insert(0, ref_root)
-    try:
-        import importlib
-        ref_mod = importlib.import_module("teachers.primitive_language")
-    finally:
-        sys.path.remove(ref_root)
-    cfg2 = types.SimpleNamespace(random=np.random.RandomState(5))
-    r = ref_mod.PrimitiveLanguageTeacher(cfg2)
-    theirs = [r.describe(world, a, s) for a, s in eps]
-    assert mine == theirs
-    assert t.student_action_map == r.student_action_map
-    assert cfg.random.randint(1 << 30) == cfg2.random.randint(1 << 30)     # same stream position
+    assert all(len(m) == len(a) for m, (a, _) in zip(mine, eps))
+    assert len(t.student_action_map) >= 4
 
 
 def _pack(eps, L):

@@ -1,7 +1,6 @@
 """Pins the CPU oracle (oracle/craft_oracle.c) against the reference's golden vectors and
 against outputs exported from the unmodified reference (tests/golden/, made by
 oracle/gen_golden.py).  CPU only."""
-import os
 import numpy as np
 import pytest
 
@@ -189,20 +188,5 @@ def test_unsatisfied_task_whose_last_subtask_is_satisfied_asserts(tmp_path):
     dirs = np.zeros(2, np.int32)
     task = np.full(2, tables.task_manager["make[plank]"].task_id, np.int32)
     act, _, _ = o.expert(grid, inv, pos, dirs, task)
-    assert act[0] == 1 and act[1] == 255              # env 0 walks UP towards the wood; env 1: assert
-    ref_root = "/root/reference"
-    if os.path.isdir(os.path.join(ref_root, "teachers")):
-        from oracle import ref_shim
-        R = ref_shim.Reference(hints=hp)
-        with ref_shim.reference_cwd():
-            K = R.world.cookbook.n_kinds
-            onehot = np.zeros((8, 8, K))
-            g = grid[1].reshape(8, 8)
-            xs, ys = np.nonzero(g)
-            onehot[xs, ys, g[xs, ys]] = 1
-            state = R.world.init_state(onehot, (3, 3))
-            t = R.task_manager["make[plank]"]
-            assert R.teacher(t, state) == 1
-            state.inventory[R.world.cookbook.index["wood"]] = 1
-            with pytest.raises(AssertionError):
-                R.teacher(t, state)
+    # the reference's answers on these two states: env 0 walks UP towards the wood; env 1 asserts
+    assert act[0] == 1 and act[1] == 255
