@@ -39,7 +39,10 @@ extern "C" {
 #define PSK_FLAG_BAD_ACTION 1   /* step(): "Unexpected action" exception, worlds/craft.py:415-416 */
 #define PSK_FLAG_INV_OVERFLOW 2 /* an inventory count would exceed 255 (u8 storage) */
 #define PSK_FLAG_BAD_LEAF 4     /* teacher: leaf is neither 'use' nor 'go', demonstration.py:18 */
-#define PSK_FLAG_OFF_GRID 8     /* agent position outside the grid */
+#define PSK_FLAG_OFF_GRID 8     /* reserved, never raised: no kernel checks the agent position.  The
+                                   Python entry points (VecCraft, HostCraft) reject positions outside
+                                   the grid; a C caller must not pass one (rows would be indexed
+                                   outside the env's grid row) */
 #define PSK_FLAG_CHAIN_TIMEOUT 16 /* fused kernels: the previous launch on the same envs never finished
                                      (aborted launch / overwritten counters); the kernel went on instead
                                      of hanging, results of that call are not to be trusted */
@@ -112,7 +115,10 @@ const char *psk_version(void);
  *   tick_variant     CTA shape of craft_tick_kernel: 0 = 64+2, 1 = 128+4, 2 = 32+1, 3 = 64+4, 4 = 32+2
  *   tick_tma, tick_persist, feat_persist, tick_pdl,
  *   step_variant     0 = tables staged in shared memory (default), 1 = read-only path, 2 = 1 + row preload
- * Unknown keys return PSK_ERR_BADARG.  Results never depend on a knob (tests/test_craft_gpu.py). */
+ * Unknown keys return PSK_ERR_BADARG.  Results never depend on a knob: tests/test_fused_states_gpu.py
+ * forces tick_variant, tick_tma, tick_persist, feat_persist, tick_pdl and rollout_variant /
+ * rollout_tma on the reference's exported states; tests/test_craft_gpu.py covers step_variant,
+ * tile_chain and the rollout variants on dataset rollouts. */
 int psk_set_tuning(const char *key, int32_t value);
 int psk_get_tuning(const char *key, int32_t *value);
 

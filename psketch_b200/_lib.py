@@ -194,6 +194,38 @@ def check_max_timesteps(max_timesteps):
     return t
 
 
+def check_agent_inputs(tables, inv=None, pos=None, dirs=None, task=None, scen_idx=None, n_scen=None):
+    """Rejects caller state that does not fit the agent record (include/psk_craft.h) before anything
+    is allocated: numpy would wrap a count or a position of 300 into the u8 record as 44, and the
+    kernels trust positions and scenario indices as row offsets (they never raise PSK_FLAG_OFF_GRID),
+    so an off-grid position or a scenario index out of range would read outside the env's rows."""
+    def bad(name, a, lo, hi):
+        a = np.asarray(a)
+        if a.size == 0:
+            return
+        if a.dtype.kind not in "iub" and not np.array_equal(a, np.floor(a)):
+            raise ValueError("%s must be whole numbers" % name)
+        if a.min() < lo or a.max() > hi:
+            raise ValueError("%s must be in %d..%d, got values in %s..%s" % (name, lo, hi, a.min(), a.max()))
+    if inv is not None:
+        inv = np.asarray(inv)
+        if inv.ndim != 2 or inv.shape[1] > min(tables.K, MAX_INV):
+            raise ValueError("inventory must be [n, <= %d], got shape %s" % (tables.K, inv.shape))
+        bad("inventory counts", inv, 0, 255)
+    if pos is not None:
+        pos = np.asarray(pos)
+        if pos.ndim != 2 or pos.shape[1] != 2:
+            raise ValueError("positions must be [n, 2], got shape %s" % (pos.shape,))
+        bad("x positions", pos[:, 0], 0, tables.W - 1)
+        bad("y positions", pos[:, 1], 0, tables.H - 1)
+    if dirs is not None:
+        bad("facing directions", dirs, 0, 3)
+    if task is not None:
+        bad("task ids", task, 0, tables.n_tasks - 1)
+    if scen_idx is not None:
+        bad("scenario indices", scen_idx, 0, n_scen - 1)
+
+
 def check(rc, what):
     if rc == PSK_OK:
         return

@@ -44,8 +44,10 @@ class HostCraft(object):
                  max_timesteps=40, chunk_envs=16384, host_threads=None):
         """host_threads: threads that widen the u8 wire frame (``features="f32_wire_u8"``), this one
         included; default min(8, cores / 2) divided among the ranks torchrun started on this box."""
-        self.lib = _lib.load()
         self.tables = tables if tables is not None else CraftTables()
+        _lib.check_agent_inputs(self.tables, pos=init_pos, dirs=init_dir, task=task, scen_idx=scen_idx,
+                                n_scen=len(scen_grids))
+        self.lib = _lib.load()
         self.ct = _lib.make_tables(self.tables)
         t = self.tables
         scen_grids = np.asarray(scen_grids, np.uint8)

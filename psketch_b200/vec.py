@@ -61,6 +61,9 @@ class VecCraft(object):
                        max_timesteps=40, device=None):
         """scen_grids u8[S, W*H] kind ids (cell (x,y) at x*H+y); scen_idx int[N]; init_pos
         int[N,2]; task int[N] (task id = 1-based position in the hint file)."""
+        tables = tables if tables is not None else CraftTables()
+        _lib.check_agent_inputs(tables, pos=init_pos, dirs=init_dir, task=task, scen_idx=scen_idx,
+                                n_scen=len(scen_grids))
         scen_grids = np.asarray(scen_grids, np.uint8)
         scen_idx = np.asarray(scen_idx, np.int32)
         n = len(scen_idx)
@@ -85,6 +88,8 @@ class VecCraft(object):
     @classmethod
     def from_states(cls, tables, grid, inv, pos, dirs, task=None, max_timesteps=40, device=None):
         """Arbitrary states (e.g. exported from the reference): every env is its own scenario."""
+        tables = tables if tables is not None else CraftTables()
+        _lib.check_agent_inputs(tables, inv=inv, pos=pos, dirs=dirs, task=task)
         grid = np.asarray(grid, np.uint8)
         n = len(grid)
         env = cls(tables, n, device=device, max_timesteps=max_timesteps)

@@ -254,8 +254,10 @@ class CraftState(object):
     @inventory.setter
     def inventory(self, value):
         self._need()
+        value = np.asarray(value)
+        _lib.check_agent_inputs(self.world.tables, inv=value.reshape(1, -1))
         self._agent = self._agent.copy()
-        self._agent[:self.world.cookbook.n_kinds] = np.asarray(value).astype(np.uint8)
+        self._agent[:self.world.cookbook.n_kinds] = value.astype(np.uint8)
         self._invalidate()
 
     @property
