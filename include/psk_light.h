@@ -36,7 +36,11 @@ typedef struct psk_light_scenario {
     uint8_t reserved[8];
 } psk_light_scenario;
 
-/* Per-env state u8[n][4]: x, y, bitmask of keys still on the map, reserved. */
+/* Per-env state u8[n][4]: x, y, bitmask of keys still on the map, reserved.
+ * Several keys may lie on one cell (the reference's dict of keys cannot hold that): one USE on the
+ * cell picks up every key lying there, in psk_light_step, the fused tick and both teachers.  A key
+ * locks its target cell only if a door stands there (worlds/light.py:233); one aimed at any other
+ * cell locks nothing. */
 #define PSK_LIGHT_STATE_BYTES 4
 
 int psk_light_reset(const psk_light_scenario *scen, const int32_t *scen_idx, uint8_t *state,
@@ -49,7 +53,9 @@ int psk_light_features(const psk_light_scenario *scen, const int32_t *scen_idx,
 int psk_light_satisfies(const psk_light_scenario *scen, const int32_t *scen_idx,
                         const uint8_t *state, uint8_t *out, int64_t n, void *stream);
 /* action u8[n] (255 = goal room unreachable, 254 = already in the goal room), dist i16[n].
- * max_keys: the largest n_keys among the scenarios used (sizes the per-warp shared memory). */
+ * max_keys: the largest n_keys among the scenarios used (sizes the per-warp shared memory).  An env
+ * whose scenario has more keys than max_keys, or whose key mask has a bit at or above its scenario's
+ * n_keys, is not searched: action 255, dist -2. */
 int psk_light_expert(const psk_light_scenario *scen, const int32_t *scen_idx,
                      const uint8_t *state, uint8_t *action, int16_t *dist, int32_t max_keys,
                      int64_t n, void *stream);
@@ -63,7 +69,14 @@ int psk_light_expert(const psk_light_scenario *scen, const int32_t *scen_idx,
  * loops of step and features in the fused tick, and by u8[1 << max_keys][32][32]: the teacher's action
  * for every state, derived from the distances when the table is built;
  * psk_light_teacher_table_bytes gives the total size.  psk_light_expert_table answers like
- * psk_light_expert (same actions, same dist). */
+ * psk_light_expert (same actions, same dist).  A scenario with more keys than max_keys gets no flood
+ * (its table says 254 in the goal room, 255 elsewhere), and a key mask with no layer in the table
+ * (mask >= 1 << max_keys: such a scenario's envs after reset, or mask bits the scenario does not
+ * have) answers 255 / dist -2 in psk_light_expert_table, psk_light_tick and psk_light_rollout;
+ * no lookup reads outside its scenario's block.
+ * Tested against oracle/light_oracle.c (tests/test_light.py on the reference's 60 scenarios,
+ * tests/test_light_limits_gpu.py on every state of generator draws of all 17 goals up to 7 keys and
+ * of synthetic scenarios up to 8 keys / 8 doors / 31 x 31 with shared doors and shared key cells). */
 int64_t psk_light_teacher_table_bytes(int64_t n_scen, int32_t max_keys);
 int psk_light_teacher_build(const psk_light_scenario *scen, int64_t n_scen, int32_t max_keys,
                             uint16_t *table, void *stream);

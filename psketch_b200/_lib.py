@@ -226,6 +226,47 @@ def check_agent_inputs(tables, inv=None, pos=None, dirs=None, task=None, scen_id
         bad("scenario indices", scen_idx, 0, n_scen - 1)
 
 
+def check_light_inputs(board, n_keys, scen_idx, state=None):
+    """Rejects Light envs that the kernels (include/psk_light.h) would read outside their tables
+    for, before anything reaches the device.  ``board`` i32[S, 2] = board_w, board_h and ``n_keys``
+    i32[S] per scenario; ``scen_idx`` [n]; ``state`` [n, 4] = x, y, key mask, steps of the episode.
+    A scenario index selects a record and a table block; a position off the board, or a mask with a
+    bit for a key the scenario does not have, is no state of the scenario (the teacher table has no
+    entry for it); the step counter must leave room for one more step below 255."""
+    board = np.asarray(board).reshape(-1, 2)
+    n_keys = np.asarray(n_keys).reshape(-1)
+
+    def whole(name, a):
+        a = np.asarray(a)
+        if a.size and a.dtype.kind not in "iub" and not np.array_equal(a, np.floor(a)):
+            raise ValueError("%s must be whole numbers" % name)
+        return a.astype(np.int64)
+    si = whole("scenario indices", scen_idx).reshape(-1)
+    if si.size and (si.min() < 0 or si.max() >= len(board)):
+        raise ValueError("scenario indices must be in 0..%d, got values in %d..%d"
+                         % (len(board) - 1, si.min(), si.max()))
+    if state is None:
+        return
+    st = whole("Light states", state)
+    if st.shape != (len(si), 4):
+        raise ValueError("Light state must be [%d, 4], got shape %s" % (len(si), st.shape))
+    if st.size and (st.min() < 0 or st.max() > 255):
+        raise ValueError("Light state bytes must be in 0..255, got values in %d..%d" % (st.min(), st.max()))
+    bad = np.flatnonzero((st[:, 0] >= board[si, 0]) | (st[:, 1] >= board[si, 1]))
+    if bad.size:
+        e = bad[0]
+        raise ValueError("env %d: position (%d, %d) is off its %d x %d board"
+                         % (e, st[e, 0], st[e, 1], board[si[e], 0], board[si[e], 1]))
+    bad = np.flatnonzero(st[:, 2] >> n_keys[si])
+    if bad.size:
+        e = bad[0]
+        raise ValueError("env %d: key mask %#x has bits at or above its scenario's %d keys"
+                         % (e, st[e, 2], n_keys[si[e]]))
+    bad = np.flatnonzero(st[:, 3] >= 255)
+    if bad.size:
+        raise ValueError("env %d: step counter %d must be below 255" % (bad[0], st[bad[0], 3]))
+
+
 def check(rc, what):
     if rc == PSK_OK:
         return

@@ -38,6 +38,16 @@ __device__ __forceinline__ bool light_locked_door(const psk_light_scenario &s, i
     return false;
 }
 
+// keys whose target cell is a door: only those lock anything (light_locked_door); a key aimed at
+// any other cell is still picked up but opens nothing
+__device__ __forceinline__ uint32_t light_door_keys(const psk_light_scenario &s) {
+    uint32_t r = 0;
+    for (int k = 0; k < s.n_keys; k++)
+        for (int d = 0; d < s.n_doors; d++)
+            if (s.keys[k][2] == s.doors[d][0] && s.keys[k][3] == s.doors[d][1]) r |= 1u << k;
+    return r;
+}
+
 __global__ void __launch_bounds__(256)
 light_reset_kernel(const psk_light_scenario *__restrict__ scen, const int32_t *__restrict__ scen_idx,
                    uint8_t *__restrict__ state, const uint8_t *__restrict__ mask, int64_t n) {
@@ -162,7 +172,8 @@ light_expert_kernel(const psk_light_scenario *__restrict__ scen, const int32_t *
         const uint32_t alive = (st >> 16) & 0xFF;
         const int nk = s.n_keys;
         const int n_layers = 1 << nk;
-        if (n_layers > layer_cap) {          // scenario has more keys than the caller announced
+        // the scenario has more keys than the caller announced, or the mask names keys it does not have
+        if (n_layers > layer_cap || alive >= (uint32_t)n_layers) {
             if (lane == 0) {
                 action[e] = 255;
                 if (dist_out) dist_out[e] = -2;
@@ -178,6 +189,7 @@ light_expert_kernel(const psk_light_scenario *__restrict__ scen, const int32_t *
             goal_row = (0x3Fu << (s.goal_ry * PSK_LIGHT_ROOM)) & ~wall_row;
         // locked-door cells per layer are recomputed on the fly: door d is locked in layer m if a
         // key of m points at it
+        const uint32_t door_keys = light_door_keys(s);
         if (((py < 32) && ((__shfl_sync(FULL, goal_row, px & 31) >> py) & 1))) {
             if (lane == 0) {
                 action[e] = 254;
@@ -189,10 +201,16 @@ light_expert_kernel(const psk_light_scenario *__restrict__ scen, const int32_t *
             // a cell of the goal room that is a locked door in layer m cannot be stood on
             uint32_t lockrow = 0;
             for (int k = 0; k < nk; k++)
-                if (((m >> k) & 1) && s.keys[k][2] == lane) lockrow |= 1u << s.keys[k][3];
+                if ((((m & door_keys) >> k) & 1) && s.keys[k][2] == lane) lockrow |= 1u << s.keys[k][3];
             R[m * 32 + lane] = goal_row & ~lockrow;
             P[m * 32 + lane] = 0;
         }
+        // byte k: the keys lying on key k's cell, for the keys in this lane's row (0 for the others)
+        uint64_t same_cell = 0;
+        for (int k = 0; k < nk; k++)
+            for (int j = 0; j < nk; j++)
+                if (s.keys[k][0] == lane && s.keys[j][0] == lane && s.keys[j][1] == s.keys[k][1])
+                    same_cell |= 1ull << (8 * k + j);
         __syncwarp();
         int found = -1;
         const int max_levels = 32 * 32 + 64;
@@ -203,22 +221,22 @@ light_expert_kernel(const psk_light_scenario *__restrict__ scen, const int32_t *
                 if ((m & ~alive) != 0) continue;
                 uint32_t lockrow = 0;
                 for (int k = 0; k < nk; k++)
-                    if (((m >> k) & 1) && s.keys[k][2] == lane) lockrow |= 1u << s.keys[k][3];
+                    if ((((m & door_keys) >> k) & 1) && s.keys[k][2] == lane) lockrow |= 1u << s.keys[k][3];
                 const uint32_t pass = ~wall_row & ~lockrow;      // cells one may stand on in layer m
                 const uint32_t cur = R[m * 32 + lane];
                 P[m * 32 + lane] = cur;
                 // predecessors by a move: p -> p+delta in R, p itself passable (agent stands there)
                 const uint32_t up = __shfl_up_sync(FULL, cur, 1), dn = __shfl_down_sync(FULL, cur, 1);
                 uint32_t add = (cur << 1) | (cur >> 1) | (lane > 0 ? up : 0u) | (lane < 31 ? dn : 0u);
-                // predecessors by USE: standing on key k (in m) with R[m \ {k}] containing the cell
+                // predecessors by USE: standing on key k (in m) with R[m \ gone] containing the cell,
+                // where gone = the keys lying on that cell (one USE picks up every key of m there)
                 for (int k = 0; k < nk; k++) {
-                    if (!((m >> k) & 1)) continue;
-                    if (s.keys[k][0] == lane) {
-                        const uint32_t bit = 1u << s.keys[k][1];
-                        // lower layer as of the PREVIOUS level: layers are swept in increasing m and
-                        // m \ {k} < m was already advanced this level, so read its snapshot P
-                        if (P[(m & ~(1 << k)) * 32 + lane] & bit) add |= bit;
-                    }
+                    const uint32_t gone = (uint32_t)(same_cell >> (8 * k)) & 0xFFu;
+                    if (!((m >> k) & 1) || !gone) continue;
+                    const uint32_t bit = 1u << s.keys[k][1];
+                    // lower layer as of the PREVIOUS level: layers are swept in increasing m and
+                    // m \ gone < m was already advanced this level, so read its snapshot P
+                    if (P[(m & ~gone) * 32 + lane] & bit) add |= bit;
                 }
                 const uint32_t nxt = cur | (add & pass);
                 R[m * 32 + lane] = nxt;
@@ -356,10 +374,11 @@ __device__ __forceinline__ void light_teacher_flood(const psk_light_scenario &s,
     uint32_t goal_row = 0;
     if (lane / PSK_LIGHT_ROOM == s.goal_rx)
         goal_row = (0x3Fu << (s.goal_ry * PSK_LIGHT_ROOM)) & ~wall_row;
+    const uint32_t door_keys = light_door_keys(s);
     auto lock_row = [&](int m) {                     // locked-door cells of this lane's row in layer m
         uint32_t r = 0;
         for (int k = 0; k < nk; k++)
-            if (((m >> k) & 1) && s.keys[k][2] == lane) r |= 1u << s.keys[k][3];
+            if ((((m & door_keys) >> k) & 1) && s.keys[k][2] == lane) r |= 1u << s.keys[k][3];
         return r;
     };
     uint32_t *B0 = s_boards, *B1 = s_boards + layer_cap * 32;
@@ -432,12 +451,21 @@ __device__ __forceinline__ int light_action_from_dist(const psk_light_scenario &
 }
 
 // Teacher query against the table (thread per env): one byte load; the distance only on request.
-__device__ __forceinline__ int light_table_action(const LightAux &aux, int x, int y, uint32_t alive) {
-    return aux.act[((alive & 0xFF) * 32 + (x & 31)) * 32 + (y & 31)];
+// A key mask that has no layer in the table (a scenario with more keys than max_keys, or mask bits
+// the scenario does not have) answers 255 / dist -2, as the search kernel does, instead of reading
+// the next scenario's block or past the end of the table.  The load keeps the mask inside the table
+// and the answer is picked after it, off the address path (an early return makes the fused tick spill
+// at its 40-register budget).
+__device__ __forceinline__ int light_table_action(const LightAux &aux, int layer_cap, int x, int y,
+                                                  uint32_t alive) {
+    const int a = aux.act[((alive & (uint32_t)(layer_cap - 1)) * 32 + (x & 31)) * 32 + (y & 31)];
+    return alive < (uint32_t)layer_cap ? a : 255;
 }
-__device__ __forceinline__ int light_table_dist(const uint16_t *T, int action, int x, int y, uint32_t alive) {
+__device__ __forceinline__ int light_table_dist(const uint16_t *T, int layer_cap, int action, int x, int y,
+                                                uint32_t alive) {
     if (action == 254) return 0;
-    const int d = T[((alive & 0xFF) * 32 + (x & 31)) * 32 + (y & 31)];
+    if (alive >= (uint32_t)layer_cap) return -2;
+    const int d = T[(alive * 32 + (x & 31)) * 32 + (y & 31)];
     return d == 0xFFFF ? -1 : d;
 }
 
@@ -454,9 +482,9 @@ light_expert_table_kernel(const psk_light_scenario *__restrict__ scen, const int
         const LightAux aux(T, layer_cap);
         const int x = st & 0xFF, y = (st >> 8) & 0xFF;
         const uint32_t alive = (st >> 16) & 0xFF;
-        const int a = light_table_action(aux, x, y, alive);
+        const int a = light_table_action(aux, layer_cap, x, y, alive);
         action[e] = (uint8_t)a;
-        if (dist_out) dist_out[e] = (int16_t)light_table_dist(T, a, x, y, alive);
+        if (dist_out) dist_out[e] = (int16_t)light_table_dist(T, layer_cap, a, x, y, alive);
     }
 }
 
@@ -475,13 +503,13 @@ struct LightTickOut {
     uint32_t next;
 };
 
-__device__ __forceinline__ LightTickOut light_tick_env(const psk_light_scenario &s, const uint16_t *T,
-                                                       const LightAux &aux, uint32_t st, int action_in,
+__device__ __forceinline__ LightTickOut light_tick_env(const psk_light_scenario &s, const LightAux &aux,
+                                                       int layer_cap, uint32_t st, int action_in,
                                                        int max_timesteps) {
     LightTickOut o;
     const int x = st & 0xFF, y = (st >> 8) & 0xFF;
     const uint32_t alive = (st >> 16) & 0xFF;
-    o.ref = light_table_action(aux, x, y, alive);
+    o.ref = light_table_action(aux, layer_cap, x, y, alive);
     const int cell = (x & 31) * 32 + (y & 31);
     const float doors_here = (float)aux.doors[cell];
     const bool lk = aux.locked(x, y, alive);
@@ -579,7 +607,7 @@ light_tick_kernel(const psk_light_scenario *__restrict__ scen, const int32_t *__
             const uint16_t *T = table + (size_t)si * light_block_u16(layer_cap);
             const LightAux aux(T, layer_cap);
             const uint32_t st = reinterpret_cast<const uint32_t *>(state)[e];
-            o = light_tick_env(scen[si], T, aux, st, action_in ? (int)action_in[e] : -1, max_timesteps);
+            o = light_tick_env(scen[si], aux, layer_cap, st, action_in ? (int)action_in[e] : -1, max_timesteps);
             expert_out[e] = (uint8_t)o.ref;
             reinterpret_cast<uint32_t *>(state)[e] = o.next;
             if (done_out) done_out[e] = o.done;
@@ -620,7 +648,7 @@ light_rollout_kernel(const psk_light_scenario *__restrict__ scen, const int32_t 
             const int64_t row = (int64_t)t * n + e;
             LightTickOut o = {};
             if (live) {
-                o = light_tick_env(s, T, aux, st, action_in ? (int)action_in[row] : -1, max_timesteps);
+                o = light_tick_env(s, aux, layer_cap, st, action_in ? (int)action_in[row] : -1, max_timesteps);
                 expert_out[row] = (uint8_t)o.ref;
                 if (done_out) done_out[row] = o.done;
                 if (success_out) success_out[row] = o.success;

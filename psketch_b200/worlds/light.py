@@ -186,16 +186,20 @@ class VecLight(object):
 
     def __init__(self, scenarios, scen_idx, device=None):
         import torch
+        recs = [s.to_c() for s in scenarios]
+        self._board = np.asarray([[c.board_w, c.board_h] for c in recs], np.int64).reshape(-1, 2)
+        self._n_keys = np.asarray([c.n_keys for c in recs], np.int64)
+        _lib.check_light_inputs(self._board, self._n_keys, scen_idx)
         if not torch.cuda.is_available():
             raise _lib.PskError("VecLight needs a CUDA device (there is no CPU fallback)")
         self.torch = torch
         self.lib = _lib.load_light()
         self.device = torch.device(device or "cuda:%d" % torch.cuda.current_device())
-        arr = (LightScenarioC * len(scenarios))(*[s.to_c() for s in scenarios])
+        arr = (LightScenarioC * len(scenarios))(*recs)
         raw = np.frombuffer(bytes(arr), dtype=np.uint8).reshape(len(scenarios), ctypes.sizeof(LightScenarioC))
         self.scen = torch.from_numpy(raw.copy()).to(self.device)
         self.max_keys = max([len(s.keys) for s in scenarios] + [0])
-        self.scen_idx = torch.as_tensor(np.asarray(scen_idx, np.int32)).to(self.device)
+        self.scen_idx = scen_idx
         self.n = len(self.scen_idx)
         self.state = torch.zeros((self.n, 4), dtype=torch.uint8, device=self.device)
         self.err = torch.zeros(1, dtype=torch.int32, device=self.device)
@@ -214,8 +218,25 @@ class VecLight(object):
             x = self.torch.as_tensor(np.asarray(x, np.uint8))
         return x.to(device=self.device, dtype=self.torch.uint8).contiguous()
 
+    @property
+    def scen_idx(self):
+        return self._scen_idx
+
+    @scen_idx.setter
+    def scen_idx(self, idx):
+        """Scenario of every env; an index out of range raises ValueError (the kernels trust it)."""
+        host = idx.cpu().numpy() if self.torch.is_tensor(idx) else np.asarray(idx)
+        _lib.check_light_inputs(self._board, self._n_keys, host)
+        self._scen_idx_host = host.astype(np.int32).reshape(-1)
+        self._scen_idx = self.torch.as_tensor(self._scen_idx_host).to(self.device)
+
     def set_state(self, st):
-        self.state.copy_(self.torch.as_tensor(np.asarray(st, np.uint8)).to(self.device))
+        """u8[N, 4] = x, y, key mask, steps of the episode.  ValueError, before anything is copied, for
+        a position off the env's board, mask bits at or above its scenario's n_keys or a step byte
+        >= 255 (the teacher table has no entry for such a state)."""
+        st = np.asarray(st)
+        _lib.check_light_inputs(self._board, self._n_keys, self._scen_idx_host, st)
+        self.state.copy_(self.torch.as_tensor(st.astype(np.uint8)).to(self.device))
 
     def reset(self, mask=None):
         mask = self._u8(mask)
