@@ -219,21 +219,35 @@ int psk_craft_rollout_u8(const psk_craft_tables *t, psk_craft_state s, psk_craft
                          uint8_t *success_out, unsigned long long *stats, int32_t *err_flags,
                          void *stream);
 
-/* Scenario sampling (make_data.py:74-144, `random_free` / `sample_scenario`) with a counter-based
- * Philox4x32-10 generator: boundary ring, then place_kinds[0..n_place) in order, then the agent,
- * each at a uniformly random free cell that keeps all free cells connected and every occupied
- * interior cell next to a free cell.  scen_grid u8[n][cell_stride], init_pos u8[n][2];
- * *fail_count (device, may be NULL) counts scenarios that ran out of draws.  Scenario i uses the
- * Philox stream (seed, i + offset): results do not depend on the launch geometry or the GPU. */
+/* The Philox streams of the three sampler entry points below.  Generator: Philox4x32-10 (Salmon
+ * et al., SC'11).  Stream (seed, s) at counter start c has key = (seed lo, seed hi) and counter words
+ * (c lo, c hi, s lo, s hi); word 0 is incremented after each 4-word block, carrying into word 1 (not
+ * into the stream words).  A block's words are consumed out[3], out[2], out[1], out[0], and a draw
+ * below n is (u64(word) * n) >> 32.  random_free draws x, then y, and rejects an occupied cell.
+ * Every output depends only on (seed, stream, counter), never on the launch geometry or the GPU;
+ * oracle/sampler_oracle.c restates all of it and the tests compare it byte for byte.
+ *
+ * Shared blocks: the random actions of env e at clock t are the first word of block t of stream
+ * (seed, e), which is the block of scenario e's (t+1)-th refill (offset 0).  With equal seeds (both
+ * default to 123) the two sources are therefore correlated; generate_dataset separates its start
+ * cells from its scenarios by XOR-ing the seed. */
+
+/* Scenario sampling (make_data.py:74-144, `random_free` / `sample_scenario`): boundary ring, then
+ * place_kinds[0..n_place) in order, then the agent, each at a uniformly random free cell that keeps
+ * all free cells connected (reachable from the lowest-index free cell) and every occupied interior
+ * cell next to a free cell, 4,096 draws at most.  Kind ids must be 1..n_kinds-1.
+ * scen_grid u8[n][cell_stride] (cell x * H + y, the tail past W * H zeroed), init_pos u8[n][2].
+ * A scenario that runs out of draws keeps the items placed so far, gets init_pos (0, 0) and counts
+ * in *fail_count (device, may be NULL).  Scenario i uses stream (seed, i + offset), counter start 0. */
 int psk_craft_sample_scenarios(const psk_craft_tables *t, uint8_t *scen_grid, uint8_t *init_pos,
                                const uint8_t *place_kinds, int32_t n_place, int32_t boundary_kind,
                                uint64_t seed, uint64_t offset, int64_t n, int32_t cell_stride,
                                int32_t *fail_count, void *stream);
 
-/* Uniform random actions for off-policy rollouts: out[e] in [0, n_actions) from
- * Philox4x32-10(key = seed, counter = (e, t + *t_dev)); t_dev (device, may be NULL) lets a counter
- * that lives on the device (e.g. stats[2], the env-step count) advance the clock under CUDA-graph
- * replay. */
+/* Uniform random actions for off-policy rollouts: out[e] in [0, n_actions) (1..255 actions) is the
+ * first draw of stream (seed, e) at counter start t + *t_dev (mod 2^64): counter words 0-1 hold the
+ * clock, words 2-3 the env.  t_dev (device, may be NULL) lets a counter that lives on the device
+ * (e.g. stats[2], the env-step count) advance the clock under CUDA-graph replay. */
 int psk_random_actions(uint8_t *out, int64_t n, int32_t n_actions, uint64_t seed, uint64_t t,
                        const unsigned long long *t_dev, void *stream);
 /* The same for `ticks` consecutive clocks at once: out u8[ticks][n], row k = the actions of clock
@@ -242,7 +256,10 @@ int psk_random_actions_block(uint8_t *out, int64_t n, int32_t ticks, int32_t n_a
                              uint64_t t, const unsigned long long *t_dev, void *stream);
 
 /* Dataset instance positions (make_data.py:203-208): per group, `per_group` distinct uniformly
- * random free cells of scenario group_scen[g]; out_pos u8[n_groups][per_group][2]. */
+ * random free cells of scenario group_scen[g] (a row index the caller guarantees is in range);
+ * out_pos u8[n_groups][per_group][2].  Group g uses stream (seed, g + offset), counter start 1,
+ * 65,536 draws at most per slot; a slot that runs out is 255/255 and counts in *fail_count, and the
+ * next slot continues from the same generator state.  cell_stride >= W * H. */
 int psk_craft_sample_positions(const psk_craft_tables *t, const uint8_t *scen_grid,
                                const int32_t *group_scen, int32_t per_group, uint8_t *out_pos,
                                uint64_t seed, uint64_t offset, int64_t n_groups,

@@ -12,7 +12,9 @@
 // Bit-equality with numpy's stream is not a goal (BASELINE.json); the procedure, and therefore
 // the distribution, is the reference's.  tests/test_scenario_gpu.py checks the invariants, the
 // kind histogram, solvability of all tasks and the cell-occupancy statistics against scenarios
-// sampled by the reference itself (tests/golden/sampler_stats.npz).
+// sampled by the reference itself (tests/golden/sampler_stats.npz); tests/test_sampler_gpu.py
+// compares every output byte of the three kernels with a plain C restatement
+// (oracle/sampler_oracle.c), which tests/test_sampler_cpu.py pins to the Philox known answers.
 #include "psk_common.cuh"
 
 namespace psk {
@@ -172,8 +174,9 @@ craft_sample_positions_kernel(const uint8_t *__restrict__ scen_grid,
     }
 }
 
-// Off-policy action source (SURVEY §8(d) config 2): action[e] ~ U{0..n_actions-1} from
-// Philox(key = seed, counter = (env, t)): reproducible whatever the launch geometry.
+// Off-policy action source (SURVEY §8(d) config 2): action[e] ~ U{0..n_actions-1} from the first
+// word of Philox stream (seed, env) at counter start t (include/psk_craft.h): reproducible whatever
+// the launch geometry.
 // out u8[ticks][n]: row k holds the actions of clock t + k (ticks = 1: the plain per-tick form; a
 // block of rows feeds psk_craft_rollout's action_in, so the off-policy variant also runs `ticks`
 // ticks per launch).
@@ -247,7 +250,7 @@ int psk_craft_sample_positions(const psk_craft_tables *t, const uint8_t *scen_gr
                                int32_t cell_stride, int32_t *fail_count, void *stream) {
     if (!t || n_groups < 0 || per_group <= 0) return PSK_ERR_BADARG;
     if (n_groups == 0) return PSK_OK;
-    if (!scen_grid || !group_scen || !out_pos) return PSK_ERR_BADARG;
+    if (!scen_grid || !group_scen || !out_pos || cell_stride < t->width * t->height) return PSK_ERR_BADARG;
     cudaStream_t st = (cudaStream_t)stream;
     if (t->width == 8 && t->height == 8)
         craft_sample_positions_kernel<8, 8><<<blocks_for(n_groups), 128, 0, st>>>(

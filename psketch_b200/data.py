@@ -135,14 +135,19 @@ def default_placement(tables):
 
 
 def sample_scenarios(tables, n, seed, offset=0, device=None, place_kinds=None):
-    """n scenarios on the device: (scen_grid u8[n, cell_stride], init_pos u8[n,2], n_failed)."""
+    """n scenarios on the device: (scen_grid u8[n, cell_stride], init_pos u8[n,2], n_failed).
+    ``place_kinds``: the kind ids to place, each in 1..K-1 (0 is the empty cell: the kernel would
+    count it as occupied while the row shows it free)."""
     import torch
+    pk = default_placement(tables) if place_kinds is None else np.asarray(place_kinds).reshape(-1)
+    if pk.size and (pk.min() < 1 or pk.max() >= tables.K):
+        raise ValueError("place_kinds must be kind ids in 1..%d, got values in %s..%s"
+                         % (tables.K - 1, pk.min(), pk.max()))
     lib = _lib.load()
     ct = _lib.make_tables(tables)
     device = torch.device(device or "cuda:%d" % torch.cuda.current_device())
     cs = ((tables.W * tables.H + 63) // 64) * 64
-    pk = torch.from_numpy(default_placement(tables) if place_kinds is None
-                          else np.asarray(place_kinds, np.uint8)).to(device)
+    pk = torch.from_numpy(pk.astype(np.uint8)).to(device)
     grid = torch.empty((n, cs), dtype=torch.uint8, device=device)
     pos = torch.empty((n, 2), dtype=torch.uint8, device=device)
     fails = torch.zeros(1, dtype=torch.int32, device=device)
@@ -157,12 +162,17 @@ def sample_scenarios(tables, n, seed, offset=0, device=None, place_kinds=None):
 
 
 def sample_positions(tables, scen_grid, group_scen, per_group, seed, offset=0):
-    """per_group distinct random free cells for every group: u8[n_groups, per_group, 2]."""
+    """per_group distinct random free cells for every group: u8[n_groups, per_group, 2].
+    ``group_scen[g]`` is the row of ``scen_grid`` that group g draws from."""
     import torch
+    gs = np.asarray(group_scen).reshape(-1)
+    if gs.size and (gs.min() < 0 or gs.max() >= len(scen_grid)):
+        raise ValueError("group_scen must index the %d scenario rows, got values in %s..%s"
+                         % (len(scen_grid), gs.min(), gs.max()))
     lib = _lib.load()
     ct = _lib.make_tables(tables)
     device = scen_grid.device
-    gs = torch.as_tensor(np.asarray(group_scen, np.int32)).to(device)
+    gs = torch.as_tensor(gs.astype(np.int32)).to(device)
     out = torch.empty((len(gs), per_group, 2), dtype=torch.uint8, device=device)
     fails = torch.zeros(1, dtype=torch.int32, device=device)
     with torch.cuda.device(device):
