@@ -10,7 +10,8 @@ models on the device.
 Per iteration, the reference's algorithm on a batch of training instances:
   instruct   the teacher's words for the instance's reference actions (``instruct_batch``)
   pass 1     the INSTRUCTED model (conditioned on those words) explores: sampled actions from the
-             episode starts, every action executed, the agent records kept (``language_decode``)
+             episode starts, every action executed, the agent records kept (``GraphedDecode``: the
+             whole pass is one CUDA graph, one step-then-observe env launch per timestep)
   describe   the teacher names what the executed actions did (``describe_batch``: position /
              inventory deltas -> words, with its stateful student-action map and random fallback)
   receive    the instructed model, conditioned on the DESCRIPTIONS, re-scores the visited states;
@@ -19,6 +20,8 @@ Per iteration, the reference's algorithm on a batch of training instances:
   imitate    the MAIN model (conditioned on the task only) re-scores pass 2's states; targets =
              pass 2's actions (:128-137);  loss = instructed + main, one AdamW step (:180-193)
 Evaluation = the main model, greedy, on the whole dev split (2,200 instances, one batch).
+The three decoding passes (pass 1, pass 2, evaluation) run as CUDA graphs (GraphedDecode);
+tests/test_language_graph_gpu.py pins them to the eager psketch_b200.rollout.language_decode.
 """
 import argparse
 import json
@@ -35,8 +38,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "examples"))
 
 from train_dagger import Batches, load_split  # noqa: E402
-from psketch_b200.rollout import language_decode  # noqa: E402
-from psketch_b200.students import Seq2SeqPolicy, task_tokens  # noqa: E402
+from psketch_b200.students import GraphedDecode, Seq2SeqPolicy, task_tokens  # noqa: E402
 from psketch_b200.tables import CraftTables  # noqa: E402
 from psketch_b200.teachers.primitive_language import ACTION_WORDS, PrimitiveLanguageTeacher, instruct_batch  # noqa: E402
 from psketch_b200.vec import VecCraft  # noqa: E402
@@ -44,26 +46,46 @@ from psketch_b200.vec import VecCraft  # noqa: E402
 T_MAX = 40
 
 
-class Recorder(object):
-    """``policy(features, t)`` for language_decode: one decoder step of ``model`` on the env's device
-    feature tensor, the action sampled (training) or arg-maxed on the device; keeps the feature frames
-    it was shown, which are the inputs of the learning passes (student.state_seqs)."""
+class DecodeStep(object):
+    """``policy(features, t)`` for GraphedDecode: one decoder step of ``model`` at time index t (the
+    language student advances time, students/primitive_language.py), reading only static tensors.
+    ``load(mem)`` copies the encoder memory into the static tensors of its shape before a replay and
+    draws the sampling noise; actions are Gumbel-max samples over that noise (exploring) or the
+    argmax (greedy)."""
 
-    def __init__(self, model, n, n_features, device, greedy):
+    def __init__(self, model, n, device, greedy):
         self.model, self.greedy = model, greedy
-        self.feats = torch.empty((T_MAX, n, n_features), dtype=torch.float32, device=device)
         self.time = torch.arange(T_MAX, device=device).unsqueeze(1).expand(T_MAX, n).contiguous()
+        self.noise = torch.zeros((T_MAX, n, model.n_actions), dtype=torch.float32, device=device)
+        self.static = {}            # encoder memories by shape (instruction length): one graph each
+        self.mem = self.state = None
 
-    def start(self, mem):
-        self.mem, self.state = mem, (mem["h0"], mem["c0"])
+    def load(self, mem):
+        """Returns the key of the graph that reads the static copy of ``mem``."""
+        key = tuple(None if v is None else tuple(v.shape) for v in mem.values())
+        if key not in self.static:
+            self.static[key] = {k: None if v is None else v.clone() for k, v in mem.items()}
+        else:
+            for k, v in mem.items():
+                if v is not None:
+                    self.static[key][k].copy_(v)
+        self.mem = self.static[key]
+        if not self.greedy:
+            self.noise.uniform_(1e-20, 1.0)
+        return key
 
     def __call__(self, features, t):
-        self.feats[t].copy_(features)
-        with torch.no_grad():
-            logits, self.state = self.model.decode_step(features, self.time[t], self.state, self.mem)
+        if t == 0:
+            self.state = (self.mem["h0"], self.mem["c0"])
+        logits, self.state = self.model.decode_step(features, self.time[t], self.state, self.mem)
         if self.greedy:
             return logits.argmax(dim=1)
-        return torch.multinomial(F.softmax(logits, dim=1), 1).squeeze(1)
+        return (logits - torch.log(-torch.log(self.noise[t]))).argmax(dim=1)     # Gumbel-max sample
+
+
+def decode(dec, mem):
+    """One decoding pass of ``dec`` (a GraphedDecode over a DecodeStep) conditioned on ``mem``."""
+    return dec.run(dec.policy.load(mem))
 
 
 def sequence_loss(logits, actions):
@@ -89,12 +111,11 @@ def evaluate(main, tables, split, device, cache={}):
     if key not in cache:
         env = VecCraft.from_instances(tables, split["grids"], split["inst_env"], split["inst_pos"],
                                       split["inst_task"], max_timesteps=255, device=device)
-        cache[key] = (env, Recorder(main, env.n, env.n_features, device, greedy=True))
-    env, rec = cache[key]
+        cache[key] = (env, GraphedDecode(env, DecodeStep(main, env.n, device, greedy=True), T_MAX, record=False))
+    env, dec = cache[key]
     main.eval()
     with torch.no_grad():
-        rec.start(main.encode(task_tokens(tables, env.task, reverse=False)))
-    language_decode(env, rec, T_MAX, record=False)
+        decode(dec, main.encode(task_tokens(tables, env.task, reverse=False)))
     main.train()
     return float((env.satisfies() == 1).float().mean())
 
@@ -113,8 +134,8 @@ def train(args):
     opt = torch.optim.AdamW(list(instructed.parameters()) + list(main.parameters()), lr=args.lr)
     teacher = PrimitiveLanguageTeacher()
     teacher.random = np.random.RandomState(args.seed)
-    explore = Recorder(instructed, args.batch, 404, device, greedy=False)
-    follow = Recorder(instructed, args.batch, 404, device, greedy=True)
+    explore = GraphedDecode(data.env, DecodeStep(instructed, args.batch, device, greedy=False), T_MAX, record=True)
+    follow = GraphedDecode(data.env, DecodeStep(instructed, args.batch, device, greedy=True), T_MAX, record=False)
     log, t0 = [], time.time()
     env_steps = episodes = 0
     for it in range(args.iters):
@@ -129,8 +150,7 @@ def train(args):
         # pass 1: exploring, instructed
         instructed.train()
         with torch.no_grad():
-            explore.start(instructed.encode(instr_tok, instr_mask))
-        first = language_decode(env, explore, T_MAX, record=True)
+            first = decode(explore, instructed.encode(instr_tok, instr_mask))
         T1 = first["timesteps"]
         L1 = int(first["lengths"].max())
         desc = teacher.describe_batch(first["actions"][:, :L1].long(), first["agents"][:L1 + 1], first["lengths"],
@@ -138,19 +158,18 @@ def train(args):
         # receive: the descriptions condition the instructed model on what it actually did
         desc_tok, desc_mask = words_to_tokens(desc, vocab, device)
         mem = instructed.encode(desc_tok, desc_mask)
-        logits = instructed.decode_sequence(explore.feats[:T1], explore.time[:T1], mem)
+        logits = instructed.decode_sequence(first["features"][:T1], explore.policy.time[:T1], mem)
         instructed_loss = sequence_loss(logits, first["actions"])
         # pass 2: greedy, original instructions, same starts
         instructed.eval()
         with torch.no_grad():
-            follow.start(instructed.encode(instr_tok, instr_mask))
-        second = language_decode(env, follow, T_MAX, record=False)
+            second = decode(follow, instructed.encode(instr_tok, instr_mask))
         instructed.train()
         T2 = second["timesteps"]
         success = env.satisfies() == 1
         # imitate: the task-conditioned model learns pass 2's behaviour
         mem = main.encode(task_tokens(tables, tasks, reverse=False))
-        logits = main.decode_sequence(follow.feats[:T2], follow.time[:T2], mem)
+        logits = main.decode_sequence(second["features"][:T2], follow.policy.time[:T2], mem)
         main_loss = sequence_loss(logits, second["actions"])
         loss = instructed_loss + main_loss
         opt.zero_grad(set_to_none=True)

@@ -177,10 +177,18 @@ int psk_craft_reset(psk_craft_state s, psk_craft_episodes ep, const uint8_t *mas
  *     action_in ? { timer -= 1; done/success/auto-reset or s = s.step(action_in[i]) } : nothing
  *     ref = teacher(task, s); f = s.features()          <- of the state AFTER the step
  * so one launch per timestep serves  a_t = policy(f_t); tick(a_t) -> f_{t+1}, ref_{t+1}, done_t.
- * In that order done_out / success_out describe the step just applied (0 when action_in is NULL). */
+ * In that order done_out / success_out describe the step just applied (0 when action_in is NULL).
+ * PSK_TICK_STEP_FIRST = "step, then observe" WITHOUT the episode rules — what the language trainers
+ * need (trainers/primitive_language.py:47-70, 93-113: every action of a running env is executed, STOP
+ * is a no-op step, a finished env keeps its state for describe / satisfies):
+ *     action_in ? s = s.step(action_in[i]) : nothing      <- CraftState.step only
+ *     ref = teacher(task, s); f = s.features()          <- of the state AFTER the step
+ * The timer byte and stats are not touched; done_out / success_out (may be NULL) are written as 0.
+ * A bad action byte raises PSK_FLAG_BAD_ACTION and leaves the env as it was (as psk_craft_step). */
 #define PSK_TICK_PIPELINE 0
 #define PSK_TICK_FUSED 1
 #define PSK_TICK_ADVANCE_FIRST 2
+#define PSK_TICK_STEP_FIRST 3
 int psk_craft_tick(const psk_craft_tables *t, psk_craft_state s, psk_craft_episodes ep,
                    const uint8_t *action_in, float *features_out, uint8_t *expert_out,
                    uint8_t *done_out, uint8_t *success_out, unsigned long long *stats,
@@ -194,7 +202,7 @@ int psk_debug_chain_skip_ticket(psk_craft_state s, int64_t env, void *stream);
 
 /* psk_craft_tick with the feature rows as bytes (features_out u8[n][n_features], see
  * psk_craft_features_u8) — same fused kernel, a quarter of the output traffic; order =
- * PSK_TICK_FUSED or PSK_TICK_ADVANCE_FIRST. */
+ * PSK_TICK_FUSED, PSK_TICK_ADVANCE_FIRST or PSK_TICK_STEP_FIRST. */
 int psk_craft_tick_u8(const psk_craft_tables *t, psk_craft_state s, psk_craft_episodes ep,
                       const uint8_t *action_in, uint8_t *features_out, uint8_t *expert_out,
                       uint8_t *done_out, uint8_t *success_out, unsigned long long *stats,

@@ -31,6 +31,7 @@ CRAFT_EXPORTS = (
     "psk_debug_wire_split_next",
 )
 FEATURES_NONE, FEATURES_F32, FEATURES_U8, FEATURES_F32_WIRE_U8 = 0, 1, 2, 3
+TICK_PIPELINE, TICK_FUSED, TICK_ADVANCE_FIRST, TICK_STEP_FIRST = 0, 1, 2, 3   # psk_craft_tick orders
 
 
 class CraftTablesC(ctypes.Structure):

@@ -1624,8 +1624,14 @@ craft_advance_kernel(const psk_craft_tables *__restrict__ T, uint8_t *__restrict
 // every CTA instead of alternating.
 // OUT = float: the reference's f32 feature rows; OUT = uint8_t: the compact byte frame
 // (psk_craft_tick_u8 / psk_craft_rollout_u8; vector-store path only: the tile IS the frame).
-template <int W, int H, int WIN, int NE, int NFW, int KC, bool USE_TMA, typename OUT = float>
-__global__ void __launch_bounds__(NE + NFW * 32)
+// STEP_FIRST: PSK_TICK_STEP_FIRST, a separate instantiation so that the other orders' code is
+// exactly what it was without it.  On 10 x 10 grids it is held to 80 registers, the budget of the
+// other orders' instantiations there (left alone, ptxas takes up to 126 and fits 4 CTAs per SM
+// instead of 6).
+template <int W, int H, int WIN, int NE, int NFW, int KC, bool USE_TMA, typename OUT = float,
+          bool STEP_FIRST = false>
+__global__ void __launch_bounds__(NE + NFW * 32,
+                                  STEP_FIRST && W * H > 64 ? 65536 / ((NE + NFW * 32) * 80) : 0)
 craft_tick_kernel(const psk_craft_tables *__restrict__ T, uint8_t *__restrict__ grid,
                   uint8_t *__restrict__ agent, const uint8_t *__restrict__ action_in,
                   const uint8_t *__restrict__ scen_grid, const int32_t *__restrict__ scen_idx,
@@ -1634,6 +1640,7 @@ craft_tick_kernel(const psk_craft_tables *__restrict__ T, uint8_t *__restrict__ 
                   uint8_t *__restrict__ success_out, unsigned long long *stats,
                   int32_t *err_flags, int64_t n, int cell_stride, int K, int nf, int adv_first,
                   uint32_t *chain, int64_t chain_g0) {
+    if constexpr (STEP_FIRST) adv_first = 1;
     constexpr int NT = NE + NFW * 32;
     constexpr int TPE = 8, EPW = 32 / TPE;
     constexpr int SPW = NE / NFW;              // env slots per feature warp
@@ -1702,8 +1709,9 @@ craft_tick_kernel(const psk_craft_tables *__restrict__ T, uint8_t *__restrict__ 
         }
         __syncthreads();
         if (adv_first) {
-            // "step, then observe" (PSK_TICK_ADVANCE_FIRST): the env threads apply action_in to the
-            // tile in shared memory first — the teacher and the feature warps then see the NEW state
+            // "step, then observe" (PSK_TICK_ADVANCE_FIRST, or PSK_TICK_STEP_FIRST without the episode
+            // rules): the env threads apply action_in to the tile in shared memory first — the teacher
+            // and the feature warps then see the NEW state
             if (env_warp && tid < ne_sp) {
                 const int64_t e = e_base + tid;
                 bool done = false, success = false;
@@ -1717,9 +1725,12 @@ craft_tick_kernel(const psk_craft_tables *__restrict__ T, uint8_t *__restrict__ 
                     const Agent before = a;
                     uint8_t *srow_w = s_rows + tid * CP;
                     const int act = action_in[e];
-                    done = advance_env<W, H>(st, a, srow_w, srow_w, act,
-                                             scen_grid + (int64_t)scen_idx[e] * CP,
-                                             init_agent + e * PSK_AGENT_BYTES, CP, success, flags);
+                    if constexpr (STEP_FIRST)   // CraftState.step only: no timer, no done, no auto-reset
+                        step_env<W, H>(st, a, srow_w, srow_w, act, flags);
+                    else
+                        done = advance_env<W, H>(st, a, srow_w, srow_w, act,
+                                                 scen_grid + (int64_t)scen_idx[e] * CP,
+                                                 init_agent + e * PSK_AGENT_BYTES, CP, success, flags);
                     bool changed = false;
 #pragma unroll
                     for (int i = 0; i < 8; i++) changed |= a.w[i] != before.w[i];
@@ -1737,7 +1748,7 @@ craft_tick_kernel(const psk_craft_tables *__restrict__ T, uint8_t *__restrict__ 
                 }
                 if (done_out) done_out[e] = done;
                 if (success_out) success_out[e] = success;
-                add_stats(stats, done, success, action_in != nullptr);
+                if constexpr (!STEP_FIRST) add_stats(stats, done, success, action_in != nullptr);
             }
             __syncthreads();
         }
@@ -2259,14 +2270,21 @@ template <int W, int H, int WIN> struct Config {
         constexpr int EPW = 32 / TPE;
         const int f = nf(t);
         const size_t smem = (size_t)NFW * feature_buffer_bytes(TMA, EPW, f, PSK_ESZ_FUSED_KERNELS);
-        auto kern = t->n_kinds == 21 ? craft_tick_kernel<W, H, WIN, NE, NFW, 21, TMA, OUT>
-                                     : craft_tick_kernel<W, H, WIN, NE, NFW, 0, TMA, OUT>;
+        auto kern = adv_first == 2
+                        ? (t->n_kinds == 21 ? craft_tick_kernel<W, H, WIN, NE, NFW, 21, TMA, OUT, true>
+                                            : craft_tick_kernel<W, H, WIN, NE, NFW, 0, TMA, OUT, true>)
+                        : (t->n_kinds == 21 ? craft_tick_kernel<W, H, WIN, NE, NFW, 21, TMA, OUT>
+                                            : craft_tick_kernel<W, H, WIN, NE, NFW, 0, TMA, OUT>);
         static size_t configured_on[PSK_MAX_DEVICES] = {0};   // the attribute is per device
         size_t &configured = configured_on[current_device()];
         if (configured != smem) {
             if (cudaFuncSetAttribute(craft_tick_kernel<W, H, WIN, NE, NFW, 21, TMA, OUT>,
                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
                 cudaFuncSetAttribute(craft_tick_kernel<W, H, WIN, NE, NFW, 0, TMA, OUT>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
+                cudaFuncSetAttribute(craft_tick_kernel<W, H, WIN, NE, NFW, 21, TMA, OUT, true>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
+                cudaFuncSetAttribute(craft_tick_kernel<W, H, WIN, NE, NFW, 0, TMA, OUT, true>,
                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
                 return PSK_ERR_CUDA;
             configured = smem;
@@ -2563,6 +2581,12 @@ int psk_craft_reset(psk_craft_state s, psk_craft_episodes ep, const uint8_t *mas
     return check(cudaGetLastError());
 }
 
+// craft_tick_kernel's adv_first argument for a tick order: 0 = observe, then advance (PSK_TICK_FUSED);
+// 1 = advance, then observe (PSK_TICK_ADVANCE_FIRST); 2 = step, then observe (PSK_TICK_STEP_FIRST)
+static int tick_order_arg(int order) {
+    return order == PSK_TICK_ADVANCE_FIRST ? 1 : order == PSK_TICK_STEP_FIRST ? 2 : 0;
+}
+
 int psk_craft_tick(const psk_craft_tables *t, psk_craft_state s, psk_craft_episodes ep,
                    const uint8_t *action_in, float *features_out, uint8_t *expert_out,
                    uint8_t *done_out, uint8_t *success_out, unsigned long long *stats,
@@ -2572,13 +2596,17 @@ int psk_craft_tick(const psk_craft_tables *t, psk_craft_state s, psk_craft_episo
     if (!expert_out || !ep.scen_grid || !ep.scen_idx || !ep.init_agent) return PSK_ERR_BADARG;
     if (features_out && (reinterpret_cast<uintptr_t>(features_out) & 15)) return PSK_ERR_BADARG;
     cudaStream_t st = (cudaStream_t)stream;
-    const int adv_first = fused == PSK_TICK_ADVANCE_FIRST;
+    const int adv_first = tick_order_arg(fused);
     if (fused && t->width * t->height <= 128) {
         PSK_DISPATCH(t, tick_fused(t, s, ep, action_in, features_out, expert_out, done_out,
                                    success_out, stats, err_flags, st, adv_first));
     }
     if (adv_first) {        // step, then observe — as separate launches (grids above 128 cells)
-        if (action_in) {
+        if (action_in && adv_first == 2) {      // CraftState.step only; done / success stay 0
+            const int rc = psk_craft_step(t, s, action_in, nullptr, nullptr, err_flags, stream);
+            if (rc) return rc;
+        }
+        if (action_in && adv_first == 1) {
             int rc = PSK_ERR_UNSUPPORTED;
             do {
                 if (Medium::matches(t)) { rc = Medium::advance(t, s, ep, action_in, done_out, success_out, stats, err_flags, st); break; }
@@ -2631,7 +2659,7 @@ int psk_craft_tick_u8(const psk_craft_tables *t, psk_craft_state s, psk_craft_ep
     if (!expert_out || !features_out || !ep.scen_grid || !ep.scen_idx || !ep.init_agent) return PSK_ERR_BADARG;
     if (reinterpret_cast<uintptr_t>(features_out) & 3) return PSK_ERR_BADARG;
     cudaStream_t st = (cudaStream_t)stream;
-    const int adv_first = order == PSK_TICK_ADVANCE_FIRST;
+    const int adv_first = tick_order_arg(order);
     if (t->width * t->height <= 128)
         PSK_DISPATCH(t, tick_u8(t, s, ep, action_in, features_out, expert_out, done_out, success_out, stats,
                                 err_flags, st, adv_first));

@@ -8,6 +8,9 @@ straight into the env kernel; one whole rollout (40 timesteps of: fused tick in 
 observe" order -> decode -> sample) is ONE CUDA graph replay with no host round trip
 (``GraphedRollout``).
 
+``GraphedDecode`` does the same for the language trainers' decoding passes (step, then observe,
+without the imitation trainer's episode rules).
+
 ``Seq2SeqPolicy`` has the architecture of the reference's ``models/lstm_seq2seq.py:LSTMSeq2SeqModel``
 (task-token encoder LSTM with source-position embeddings, decoder LSTM over [features, time
 embedding], dot-product attention over the encoder outputs, two-layer predictor), organised for
@@ -218,16 +221,99 @@ class GraphedRollout(object):
             self._body()
             return self
         if self.graph is None:
-            self._body()                                # warm-up: allocations, cuDNN plans, tables
-            env.reset()
-            torch.cuda.synchronize()
-            side = torch.cuda.Stream(device=env.device)
-            side.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(side):
-                self.graph = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(self.graph, stream=side):
-                    self._body()
-            torch.cuda.current_stream().wait_stream(side)
-            env.reset()
+            self.graph = capture_graph(env, self._body)
         self.graph.replay()
         return self
+
+
+def capture_graph(env, body):
+    """``body`` captured as one CUDA graph.  A warm-up run first (allocations, cuDNN plans, and the
+    first call with the env's tables outside the capture), then the capture on a side stream; leaves
+    the envs at their episode starts."""
+    body()
+    env.reset()
+    torch.cuda.synchronize()
+    side = torch.cuda.Stream(device=env.device)
+    side.wait_stream(torch.cuda.current_stream())
+    with torch.cuda.stream(side):
+        graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(graph, stream=side):
+            body()
+    torch.cuda.current_stream().wait_stream(side)
+    env.reset()
+    return graph
+
+
+class GraphedDecode(object):
+    """psketch_b200.rollout.language_decode — one decoding pass of the language trainers
+    (trainers/primitive_language.py:47-70, 93-113) from the envs' episode starts — as ONE CUDA graph:
+    T + 1 step-then-observe ticks (``VecCraft.step_observe``: CraftState.step alone, every action of a
+    running env executed, STOP a no-op, finished envs keep their state), the first without actions,
+    and per timestep ``policy(features, t) -> actions [N]``, any capturable callable that reads only
+    tensors whose addresses do not change between replays.  The bookkeeping of language_decode runs
+    as device ops; nothing crosses PCIe inside a replay.
+
+    ``run(key)`` returns what language_decode returns — actions u8[N, T] padded with 255, lengths
+    i64[N], agents u8[L + 1, N, 32] (None unless ``record``), steps — plus ``features``, the frames
+    the policy saw (f32[T, N, F]).  The pass always runs T timesteps and ``timesteps`` is
+    lengths.max() (language_decode rounds up to its polling interval; timesteps where no env runs
+    add nothing to the trainers' losses).  One graph is kept per ``key``: a policy whose static
+    tensors change shape (instructions of another length) gives each shape its own key."""
+
+    def __init__(self, env, policy, max_timesteps=40, record=True, use_graph=True):
+        from . import _lib
+        self.env, self.policy, self.T = env, policy, _lib.check_max_timesteps(max_timesteps)
+        self.record, self.use_graph = record, use_graph
+        n, dev = env.n, env.device
+        self.feats = torch.zeros((self.T + 1, n, env.n_features), dtype=torch.float32, device=dev)
+        self.acts = torch.full((n, self.T), 255, dtype=torch.uint8, device=dev)
+        self.lengths = torch.zeros(n, dtype=torch.long, device=dev)
+        self.agents = torch.zeros((self.T + 1, n, env.agent.shape[1]), dtype=torch.uint8, device=dev) if record else None
+        self.done = torch.zeros(n, dtype=torch.bool, device=dev)
+        self.steps = torch.zeros((), dtype=torch.long, device=dev)
+        self.out = {}
+        self.graphs = {}
+
+    def _body(self):
+        env, T = self.env, self.T
+        self.done.zero_()
+        self.lengths.zero_()
+        self.steps.zero_()
+        self.acts.fill_(255)
+        if self.record:
+            self.agents[0].copy_(env.agent)
+        prev = None
+        for t in range(T + 1):
+            # ONE env launch per timestep: the previous actions (none at t = 0), then the features of
+            # the new states (frame T, of the final states, is seen by nobody)
+            env.step_observe(actions=prev, features_out=self.feats[t], out=self.out)
+            if self.record and t > 0:
+                self.agents[t].copy_(env.agent)
+            if t == T:
+                break
+            a = self.policy(self.feats[t], t).to(torch.uint8)
+            live = ~self.done
+            self.acts[:, t] = torch.where(live, a, self.acts[:, t])
+            prev = torch.where(live, a, torch.full_like(a, STOP))      # finished envs idle
+            self.steps += live.sum()
+            self.lengths += live
+            self.done |= (a == STOP) | (t == T - 1)
+
+    @torch.no_grad()
+    def run(self, key=None):
+        from . import _lib
+        env = self.env
+        env.reset()
+        if not self.use_graph:
+            self._body()
+        else:
+            if key not in self.graphs:
+                self.graphs[key] = capture_graph(env, self._body)
+            self.graphs[key].replay()
+        # the pass does not use the teacher's labels that come with every tick: the teacher's assertion
+        # (FLAG_BAD_LEAF, a state where the reference's teacher would raise) is not an error of the pass
+        env.err_flags.bitwise_and_(~_lib.FLAG_BAD_LEAF)
+        env.check_errors()
+        L = int(self.lengths.max().item())
+        return dict(actions=self.acts, lengths=self.lengths, agents=self.agents[:L + 1] if self.record else None,
+                    steps=int(self.steps.item()), timesteps=L, features=self.feats[:self.T])

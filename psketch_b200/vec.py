@@ -236,6 +236,28 @@ class VecCraft(object):
         _lib.check(rc, "psk_craft_tick")
         return out
 
+    def step_observe(self, actions=None, features_out=None, out=None):
+        """One launch of PSK_TICK_STEP_FIRST: ``actions`` (None = no step) go through CraftState.step
+        alone — no timer, no done, no auto-reset, STOP is the idle action — then the teacher's action
+        and the features of the NEW states.  The language trainers' decoding step
+        (trainers/primitive_language.py:47-70).  A ``features_out`` tensor of dtype uint8 selects the
+        byte frame.  Returns dict(expert u8[N], features)."""
+        actions = self._u8(actions)
+        if out is None:
+            out = {}
+        if "expert" not in out:
+            out["expert"] = torch.empty(self.n, dtype=torch.uint8, device=self.device)
+        if features_out is None:
+            features_out = torch.empty((self.n, self.n_features), dtype=torch.float32, device=self.device)
+        out["features"] = features_out
+        entry = self.lib.psk_craft_tick_u8 if features_out.dtype == torch.uint8 else self.lib.psk_craft_tick
+        with torch.cuda.device(self.device):
+            rc = entry(ctypes.byref(self.ct), self._state(), self._episodes(), _ptr(actions),
+                       _ptr(features_out), _ptr(out["expert"]), None, None, None, _ptr(self.err_flags),
+                       _lib.TICK_STEP_FIRST, self._stream())
+        _lib.check(rc, "psk_craft_tick")
+        return out
+
     def rollout(self, ticks, actions=None, features_out=None, out=None, want_flags=True):
         """``ticks`` rollout ticks in one launch (psk_craft_rollout).  actions: u8[ticks, N] or None
         (follow the teacher); features_out: f32[R, N, n_features] ring or None.  Returns
