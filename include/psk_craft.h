@@ -14,6 +14,15 @@
  * asynchronous on that stream.  Kernel-detected conditions that make the reference raise are
  * OR-ed into `*err_flags` (device int32, may be NULL) as PSK_FLAG_* bits.
  *
+ * Domain: 1 <= width, height <= 64 (the agent record stores x and y as bytes; the teacher's boards
+ * hold 64 rows of 64 cells), window_w and window_h odd from 1 to 9, 1 <= n_kinds <= 24.  Even windows
+ * are outside it: the pooled window has ww^2 + 1 cells per axis, which the reference's block_reduce pads
+ * and its features() then rejects by its own length check.  Five geometries have specialised kernels
+ * (8x8 / 3, 10x10 / 5 and 16x16, 32x32, 64x64 with a 3x3 window, fused tick and rollout kernels up to
+ * 128 cells); every other one runs the generic tier (psk_craft_generic.cu), which reads the geometry
+ * from the tables at run time and serves the tick and rollout entry points as separate launches.
+ * Same results either way.  Tables outside the domain: PSK_ERR_UNSUPPORTED.
+ *
  * Device state layout (one env = one row in each array):
  *   grid  u8[n][cell_stride]   kind id per cell, 0 = free, cell (x, y) at x*height + y
  *                              (the reference's one-hot float64 grid[x, y, kind], craft.py:275-283);
@@ -32,7 +41,7 @@ extern "C" {
 #endif
 
 #define PSK_OK 0
-#define PSK_ERR_UNSUPPORTED 1 /* (width, height, window) combination not built */
+#define PSK_ERR_UNSUPPORTED 1 /* tables outside the domain below */
 #define PSK_ERR_BADARG 2
 #define PSK_ERR_CUDA 3
 
@@ -115,6 +124,7 @@ const char *psk_version(void);
  *   tick_variant     CTA shape of craft_tick_kernel: 0 = 64+2, 1 = 128+4, 2 = 32+1, 3 = 64+4, 4 = 32+2
  *   tick_tma, tick_persist, feat_persist, tick_pdl,
  *   step_variant     0 = tables staged in shared memory (default), 1 = read-only path, 2 = 1 + row preload
+ *   generic          1 = the five built geometries take the generic tier too (no fused tick / rollout)
  * Unknown keys return PSK_ERR_BADARG.  Results never depend on a knob: tests/test_fused_states_gpu.py
  * forces tick_variant, tick_tma, tick_persist, feat_persist, tick_pdl and rollout_variant /
  * rollout_tma on the reference's exported states; tests/test_craft_gpu.py covers step_variant,
@@ -122,7 +132,8 @@ const char *psk_version(void);
 int psk_set_tuning(const char *key, int32_t value);
 int psk_get_tuning(const char *key, int32_t *value);
 
-/* number of bytes of one feature row, or -1 when the configuration is unsupported */
+/* number of features of one row (2 * window_w * window_h * n_kinds + n_kinds + 5), or -1 when the
+ * tables are outside the domain; psk_craft_supported: 1 inside the domain, else 0 */
 int psk_craft_n_features(const psk_craft_tables *t);
 int psk_craft_supported(const psk_craft_tables *t);
 

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.dirname(HERE)
 LIB = os.path.join(PKG, "libpsk_b200.so")
-SOURCES = ["psk_craft.cu", "psk_scenario.cu", "psk_light.cu", "psk_host.cu", "psk_hostcpu.cpp"]
+SOURCES = ["psk_craft.cu", "psk_craft_generic.cu", "psk_scenario.cu", "psk_light.cu", "psk_host.cu", "psk_hostcpu.cpp"]
 HEADERS = ["psk_common.cuh", "psk_hostcpu.h", os.path.join("..", "..", "include", "psk_craft.h"),
            os.path.join("..", "..", "include", "psk_light.h")]
 

@@ -125,6 +125,54 @@ __device__ __forceinline__ void store_agent(uint8_t *agent, int64_t e, const Age
 }
 
 // ---------------------------------------------------------------------------------------------
+// satisfies (worlds/craft.py:285-294) and the hint-tree walk (teachers/base.py:10-25), shared by the
+// specialised kernels (psk_craft.cu) and the run-time-geometry ones (psk_craft_generic.cu).
+__device__ __forceinline__ int node_satisfied(uint32_t nd, const Agent &a, int facing) {
+    const int sat = nd & 0xFF, arg = (nd >> 8) & 0xFF;
+    if (sat == SAT_INV) return arg < PSK_MAX_INV ? (a.inv(arg) > 0) : 0;
+    if (sat == SAT_FACING) return facing == arg;
+    return 2;  // None
+}
+
+// first incomplete leaf of `task` (node word), or 0 when there is none (-> STOP).
+// WARP-CONVERGENT: all 32 lanes call it together; the loop runs in lock-step (vote) so that the
+// lanes are converged again when it ends, whatever their individual trip counts were.
+__device__ __forceinline__ uint32_t find_incomplete(const SharedTables &st, int task,
+                                                    const Agent &a, int facing) {
+    const int n = st.task_len(task);
+    int i = 0;
+    uint32_t leaf = 0;
+    while (__any_sync(0xffffffffu, i < n && !leaf)) {
+        if (i < n && !leaf) {
+            const uint32_t nd = st.node(task, i);
+            if (node_satisfied(nd, a, facing) == 1) {
+                // bit 0x40 of the leaf byte: last subtask of an (unsatisfied) task — the reference's
+                // assert at teachers/base.py:23-24; reported like a bad leaf
+                if (nd & 0x00400000u) leaf = (uint32_t(LEAF_BAD) << 16) | 0x80000000u;
+                i = nd >> 24;
+            } else if ((nd >> 16) & 0x0F) leaf = nd | 0x80000000u;  // bit 31 marks "found"
+            else i++;
+        }
+    }
+    return leaf;
+}
+
+// episode / success / env-step counters of a rollout tick, one atomic per warp and counter
+__device__ __forceinline__ void add_stats(unsigned long long *stats, bool done, bool success,
+                                          bool counted) {
+    const unsigned full = __activemask();
+    const int n_done = __popc(__ballot_sync(full, done));
+    const int n_succ = __popc(__ballot_sync(full, success));
+    const int n_step = __popc(__ballot_sync(full, counted));
+    const int leader = __ffs(full) - 1;
+    if (stats && (int)(threadIdx.x & 31) == leader) {
+        if (n_done) atomicAdd(stats + 0, (unsigned long long)n_done);
+        if (n_succ) atomicAdd(stats + 1, (unsigned long long)n_succ);
+        if (n_step) atomicAdd(stats + 2, (unsigned long long)n_step);
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
 // Bitboards over the grid: bit (x*H + y).  uint64_t for W*H <= 64, unsigned __int128 up to 128.
 template <int CELLS> struct BoardOf { using type = unsigned __int128; };
 template <> struct BoardOf<64> { using type = uint64_t; };
@@ -234,5 +282,29 @@ static inline int current_device() {
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= PSK_MAX_DEVICES) dev = 0;
     return dev;
 }
+
+// ---------------------------------------------------------------------------------------------
+// Generic tier (psk_craft_generic.cu): the primitives for any geometry of the generic domain
+// (include/psk_craft.h), geometry and K read from the device tables `dt` at run time.  `grid` is
+// the launch's CTA count: step, satisfies and advance run 256-thread CTAs of one env per thread,
+// expert, find_closest and features 128-thread CTAs of one env per warp.  Launches are
+// asynchronous on `st`; the return value is a PSK_* code.
+constexpr int GENERIC_THREAD_CTA = 256, GENERIC_WARP_CTA = 128;
+int generic_step(int grid, const psk_craft_tables *dt, psk_craft_state s, const uint8_t *action,
+                 const uint8_t *active, float *reward, int32_t *err, cudaStream_t st);
+int generic_satisfies(int grid, const psk_craft_tables *dt, psk_craft_state s, const uint8_t *task,
+                      uint8_t *out, cudaStream_t st);
+int generic_expert(int grid, const psk_craft_tables *dt, psk_craft_state s, const uint8_t *task,
+                   uint8_t *action, int16_t *dist, int32_t *err, cudaStream_t st);
+int generic_find_closest(int grid, const psk_craft_tables *dt, psk_craft_state s, const uint8_t *kind,
+                         uint8_t *goal, int16_t *len, uint8_t *seq, int seq_cap, cudaStream_t st);
+int generic_features(int grid, const psk_craft_tables *dt, psk_craft_state s, float *out_f32,
+                     uint8_t *out_u8, cudaStream_t st);
+int generic_advance(int grid, const psk_craft_tables *dt, psk_craft_state s, psk_craft_episodes ep,
+                    const uint8_t *action, uint8_t *done, uint8_t *success, unsigned long long *stats,
+                    int32_t *err, cudaStream_t st);
+// true when psk_craft_tick / _tick_u8 run the fused kernel for these tables (one of the five built
+// geometries, generic tier not forced); the host contexts' zero-copy route needs it
+bool craft_fused_built(const psk_craft_tables *t);
 
 }  // namespace psk

@@ -176,36 +176,6 @@ __device__ __forceinline__ int facing_kind(const Agent &a, const uint8_t *row) {
     return row[fx * H + fy];
 }
 
-__device__ __forceinline__ int node_satisfied(uint32_t nd, const Agent &a, int facing) {
-    const int sat = nd & 0xFF, arg = (nd >> 8) & 0xFF;
-    if (sat == SAT_INV) return arg < PSK_MAX_INV ? (a.inv(arg) > 0) : 0;
-    if (sat == SAT_FACING) return facing == arg;
-    return 2;  // None
-}
-
-// first incomplete leaf of `task` (node word), or 0 when there is none (-> STOP).
-// WARP-CONVERGENT: all 32 lanes call it together; the loop runs in lock-step (vote) so that the
-// lanes are converged again when it ends, whatever their individual trip counts were.
-__device__ __forceinline__ uint32_t find_incomplete(const SharedTables &st, int task,
-                                                    const Agent &a, int facing) {
-    const int n = st.task_len(task);
-    int i = 0;
-    uint32_t leaf = 0;
-    while (__any_sync(0xffffffffu, i < n && !leaf)) {
-        if (i < n && !leaf) {
-            const uint32_t nd = st.node(task, i);
-            if (node_satisfied(nd, a, facing) == 1) {
-                // bit 0x40 of the leaf byte: last subtask of an (unsatisfied) task — the reference's
-                // assert at teachers/base.py:23-24; reported like a bad leaf
-                if (nd & 0x00400000u) leaf = (uint32_t(LEAF_BAD) << 16) | 0x80000000u;
-                i = nd >> 24;
-            } else if ((nd >> 16) & 0x0F) leaf = nd | 0x80000000u;  // bit 31 marks "found"
-            else i++;
-        }
-    }
-    return leaf;
-}
-
 template <int W, int H>
 __global__ void __launch_bounds__(256)
 craft_satisfies_kernel(const psk_craft_tables *__restrict__ T,
@@ -1568,20 +1538,6 @@ __device__ __forceinline__ bool advance_env(const SharedTables &st, Agent &a, ui
     return done;
 }
 
-__device__ __forceinline__ void add_stats(unsigned long long *stats, bool done, bool success,
-                                          bool counted) {
-    const unsigned full = __activemask();
-    const int n_done = __popc(__ballot_sync(full, done));
-    const int n_succ = __popc(__ballot_sync(full, success));
-    const int n_step = __popc(__ballot_sync(full, counted));
-    const int leader = __ffs(full) - 1;
-    if (stats && (int)(threadIdx.x & 31) == leader) {
-        if (n_done) atomicAdd(stats + 0, (unsigned long long)n_done);
-        if (n_succ) atomicAdd(stats + 1, (unsigned long long)n_succ);
-        if (n_step) atomicAdd(stats + 2, (unsigned long long)n_step);
-    }
-}
-
 template <int W, int H>
 __global__ void __launch_bounds__(256)
 craft_advance_kernel(const psk_craft_tables *__restrict__ T, uint8_t *__restrict__ grid,
@@ -2025,10 +1981,10 @@ static int num_sms() {
 // changed at any time afterwards, so tests and A/B runs can force every kernel variant.
 enum TuneKey { TUNE_ROLLOUT_VARIANT, TUNE_ROLLOUT_TMA, TUNE_TICK_VARIANT, TUNE_TICK_TMA,
                TUNE_TICK_PERSIST, TUNE_FEAT_PERSIST, TUNE_TICK_PDL, TUNE_STEP_VARIANT,
-               TUNE_TILE_CHAIN, TUNE_COUNT };
+               TUNE_TILE_CHAIN, TUNE_GENERIC, TUNE_COUNT };
 static const char *const tune_names[TUNE_COUNT] = {
     "rollout_variant", "rollout_tma", "tick_variant", "tick_tma", "tick_persist", "feat_persist",
-    "tick_pdl", "step_variant", "tile_chain"};
+    "tick_pdl", "step_variant", "tile_chain", "generic"};
 static std::atomic<int> tune_val[TUNE_COUNT];
 static std::once_flag tune_once;
 static void tune_init() {
@@ -2466,15 +2422,99 @@ using Stress16 = Config<16, 16, 3>;  // enlarged-grid stress tests (BASELINE con
 using Stress32 = Config<32, 32, 3>;
 using Stress64 = Config<64, 64, 3>;
 
-#define PSK_DISPATCH(t, CALL)                             \
-    do {                                                  \
-        if (Medium::matches(t)) return Medium::CALL;      \
-        if (Large::matches(t)) return Large::CALL;        \
-        if (Stress16::matches(t)) return Stress16::CALL;  \
-        if (Stress32::matches(t)) return Stress32::CALL;  \
-        if (Stress64::matches(t)) return Stress64::CALL;  \
-        return PSK_ERR_UNSUPPORTED;                       \
+// Every other geometry of the generic domain (include/psk_craft.h): the run-time-geometry primitives
+// of psk_craft_generic.cu.  No fused tick or rollout kernel: psk_craft_tick / _tick_u8 / _rollout /
+// _rollout_u8 run them as the pipeline of separate launches.
+struct Generic {
+    static bool matches(const psk_craft_tables *t) {
+        const auto odd_win = [](int w) { return w >= 1 && w <= 9 && (w & 1); };
+        return t->width >= 1 && t->width <= 64 && t->height >= 1 && t->height <= 64 &&
+               odd_win(t->window_w) && odd_win(t->window_h) && t->n_kinds >= 1 && t->n_kinds <= PSK_MAX_INV;
+    }
+    static int warp_grid(int64_t n) { return grid_for(n, GENERIC_WARP_CTA / 32, 16); }
+    static int thread_grid(int64_t n) { return grid_for(n, GENERIC_THREAD_CTA, 8); }
+
+    static int step(const psk_craft_tables *t, psk_craft_state s, const uint8_t *action,
+                    const uint8_t *active, float *reward, int32_t *err, cudaStream_t st) {
+        PSK_DT(dt);
+        return generic_step(thread_grid(s.n), dt, s, action, active, reward, err, st);
+    }
+    static int satisfies(const psk_craft_tables *t, psk_craft_state s, const uint8_t *task,
+                         uint8_t *out, cudaStream_t st) {
+        PSK_DT(dt);
+        return generic_satisfies(thread_grid(s.n), dt, s, task, out, st);
+    }
+    static int expert(const psk_craft_tables *t, psk_craft_state s, const uint8_t *task,
+                      uint8_t *action, int16_t *dist, int32_t *err, cudaStream_t st) {
+        PSK_DT(dt);
+        return generic_expert(warp_grid(s.n), dt, s, task, action, dist, err, st);
+    }
+    static int find_closest(const psk_craft_tables *t, psk_craft_state s, const uint8_t *kind,
+                            uint8_t *goal, int16_t *len, uint8_t *seq, int seq_cap,
+                            cudaStream_t st) {
+        PSK_DT(dt);
+        return generic_find_closest(warp_grid(s.n), dt, s, kind, goal, len, seq, seq_cap, st);
+    }
+    static int features(const psk_craft_tables *t, psk_craft_state s, float *out, int /*impl*/,
+                        cudaStream_t st) {
+        PSK_DT(dt);
+        return generic_features(warp_grid(s.n), dt, s, out, nullptr, st);
+    }
+    static int features_u8(const psk_craft_tables *t, psk_craft_state s, uint8_t *out, cudaStream_t st) {
+        PSK_DT(dt);
+        return generic_features(warp_grid(s.n), dt, s, nullptr, out, st);
+    }
+    static int advance(const psk_craft_tables *t, psk_craft_state s, psk_craft_episodes ep,
+                       const uint8_t *action, uint8_t *done, uint8_t *success,
+                       unsigned long long *stats, int32_t *err, cudaStream_t st) {
+        PSK_DT(dt);
+        return generic_advance(thread_grid(s.n), dt, s, ep, action, done, success, stats, err, st);
+    }
+};
+
+// tuning key `generic` = 1: the five built geometries take the generic tier too (tests, A/B runs)
+static bool generic_forced() { return tune(TUNE_GENERIC) == 1; }
+
+// The specialised configuration of the tables, if any; returns from the caller.
+#define PSK_DISPATCH_BUILT(t, CALL)                           \
+    do {                                                      \
+        if (!generic_forced()) {                              \
+            if (Medium::matches(t)) return Medium::CALL;      \
+            if (Large::matches(t)) return Large::CALL;        \
+            if (Stress16::matches(t)) return Stress16::CALL;  \
+            if (Stress32::matches(t)) return Stress32::CALL;  \
+            if (Stress64::matches(t)) return Stress64::CALL;  \
+        }                                                     \
     } while (0)
+
+#define PSK_DISPATCH(t, CALL)                                 \
+    do {                                                      \
+        PSK_DISPATCH_BUILT(t, CALL);                          \
+        if (Generic::matches(t)) return Generic::CALL;        \
+        return PSK_ERR_UNSUPPORTED;                           \
+    } while (0)
+
+static bool built(const psk_craft_tables *t) {
+    return Medium::matches(t) || Large::matches(t) || Stress16::matches(t) || Stress32::matches(t) ||
+           Stress64::matches(t);
+}
+
+bool craft_fused_built(const psk_craft_tables *t) {
+    return !generic_forced() && built(t) && t->width * t->height <= 128;
+}
+
+// The specialised kernels write feature frames with 128-bit (f32) / 32-bit (u8) stores and reject frames
+// that do not start on such a boundary; the generic tier stores single elements, so its frames, whose rows
+// need not be multiples of 16 bytes (ring slots of psk_craft_rollout included), may start anywhere.
+static bool frame_misaligned(const psk_craft_tables *t, const void *frame, uintptr_t align) {
+    return (reinterpret_cast<uintptr_t>(frame) & (align - 1)) && !generic_forced() && built(t);
+}
+
+static int advance_any(const psk_craft_tables *t, psk_craft_state s, psk_craft_episodes ep,
+                       const uint8_t *action, uint8_t *done, uint8_t *success, unsigned long long *stats,
+                       int32_t *err, cudaStream_t st) {
+    PSK_DISPATCH(t, advance(t, s, ep, action, done, success, stats, err, st));
+}
 
 static bool state_ok(const psk_craft_tables *t, const psk_craft_state &s) {
     if (!t || s.n < 0) return false;
@@ -2518,8 +2558,7 @@ int psk_get_tuning(const char *key, int32_t *value) {
 
 int psk_craft_supported(const psk_craft_tables *t) {
     if (!t) return 0;
-    return Medium::matches(t) || Large::matches(t) || Stress16::matches(t) || Stress32::matches(t) ||
-           Stress64::matches(t);
+    return built(t) || Generic::matches(t);
 }
 
 int psk_craft_n_features(const psk_craft_tables *t) {
@@ -2594,27 +2633,20 @@ int psk_craft_tick(const psk_craft_tables *t, psk_craft_state s, psk_craft_episo
     if (!state_ok(t, s)) return PSK_ERR_BADARG;
     if (s.n == 0) return PSK_OK;
     if (!expert_out || !ep.scen_grid || !ep.scen_idx || !ep.init_agent) return PSK_ERR_BADARG;
-    if (features_out && (reinterpret_cast<uintptr_t>(features_out) & 15)) return PSK_ERR_BADARG;
+    if (features_out && frame_misaligned(t, features_out, 16)) return PSK_ERR_BADARG;
     cudaStream_t st = (cudaStream_t)stream;
     const int adv_first = tick_order_arg(fused);
     if (fused && t->width * t->height <= 128) {
-        PSK_DISPATCH(t, tick_fused(t, s, ep, action_in, features_out, expert_out, done_out,
-                                   success_out, stats, err_flags, st, adv_first));
+        PSK_DISPATCH_BUILT(t, tick_fused(t, s, ep, action_in, features_out, expert_out, done_out,
+                                         success_out, stats, err_flags, st, adv_first));
     }
-    if (adv_first) {        // step, then observe — as separate launches (grids above 128 cells)
+    if (adv_first) {        // step, then observe — as separate launches (grids above 128 cells, generic tier)
         if (action_in && adv_first == 2) {      // CraftState.step only; done / success stay 0
             const int rc = psk_craft_step(t, s, action_in, nullptr, nullptr, err_flags, stream);
             if (rc) return rc;
         }
         if (action_in && adv_first == 1) {
-            int rc = PSK_ERR_UNSUPPORTED;
-            do {
-                if (Medium::matches(t)) { rc = Medium::advance(t, s, ep, action_in, done_out, success_out, stats, err_flags, st); break; }
-                if (Large::matches(t)) { rc = Large::advance(t, s, ep, action_in, done_out, success_out, stats, err_flags, st); break; }
-                if (Stress16::matches(t)) { rc = Stress16::advance(t, s, ep, action_in, done_out, success_out, stats, err_flags, st); break; }
-                if (Stress32::matches(t)) { rc = Stress32::advance(t, s, ep, action_in, done_out, success_out, stats, err_flags, st); break; }
-                if (Stress64::matches(t)) { rc = Stress64::advance(t, s, ep, action_in, done_out, success_out, stats, err_flags, st); break; }
-            } while (0);
+            const int rc = advance_any(t, s, ep, action_in, done_out, success_out, stats, err_flags, st);
             if (rc) return rc;
         } else {
             if (done_out && cudaMemsetAsync(done_out, 0, (size_t)s.n, st) != cudaSuccess) return PSK_ERR_CUDA;
@@ -2631,7 +2663,7 @@ int psk_craft_tick(const psk_craft_tables *t, psk_craft_state s, psk_craft_episo
         if (rc) return rc;
     }
     const uint8_t *act = action_in ? action_in : expert_out;
-    PSK_DISPATCH(t, advance(t, s, ep, act, done_out, success_out, stats, err_flags, st));
+    return advance_any(t, s, ep, act, done_out, success_out, stats, err_flags, st);
 }
 
 // Fault injection for the tile-chaining safety net (tests only): hands out one ticket of the group that
@@ -2657,13 +2689,13 @@ int psk_craft_tick_u8(const psk_craft_tables *t, psk_craft_state s, psk_craft_ep
     if (!state_ok(t, s)) return PSK_ERR_BADARG;
     if (s.n == 0) return PSK_OK;
     if (!expert_out || !features_out || !ep.scen_grid || !ep.scen_idx || !ep.init_agent) return PSK_ERR_BADARG;
-    if (reinterpret_cast<uintptr_t>(features_out) & 3) return PSK_ERR_BADARG;
+    if (frame_misaligned(t, features_out, 4)) return PSK_ERR_BADARG;
     cudaStream_t st = (cudaStream_t)stream;
     const int adv_first = tick_order_arg(order);
     if (t->width * t->height <= 128)
-        PSK_DISPATCH(t, tick_u8(t, s, ep, action_in, features_out, expert_out, done_out, success_out, stats,
-                                err_flags, st, adv_first));
-    // grids above 128 cells: the feature kernel writes the bytes, the tick does the rest
+        PSK_DISPATCH_BUILT(t, tick_u8(t, s, ep, action_in, features_out, expert_out, done_out, success_out, stats,
+                                      err_flags, st, adv_first));
+    // grids above 128 cells and the generic tier: the feature kernel writes the bytes, the tick does the rest
     if (!adv_first) {
         const int rc = psk_craft_features_u8(t, s, features_out, stream);
         if (rc) return rc;
@@ -2682,10 +2714,10 @@ int psk_craft_rollout_u8(const psk_craft_tables *t, psk_craft_state s, psk_craft
     if (!state_ok(t, s) || ticks < 0 || !features_out || feat_ring <= 0) return PSK_ERR_BADARG;
     if (s.n == 0 || ticks == 0) return PSK_OK;
     if (!expert_out || !ep.scen_grid || !ep.scen_idx || !ep.init_agent) return PSK_ERR_BADARG;
-    if (reinterpret_cast<uintptr_t>(features_out) & 3) return PSK_ERR_BADARG;
+    if (frame_misaligned(t, features_out, 4)) return PSK_ERR_BADARG;
     cudaStream_t st = (cudaStream_t)stream;
     int rc = PSK_ERR_UNSUPPORTED;
-    if (Medium::matches(t))
+    if (Medium::matches(t) && !generic_forced())
         rc = Medium::rollout_u8(t, s, ep, ticks, action_in, features_out, feat_ring, expert_out, done_out,
                                 success_out, stats, err_flags, st);
     if (rc != PSK_ERR_UNSUPPORTED) return rc;
@@ -2709,10 +2741,10 @@ int psk_craft_rollout(const psk_craft_tables *t, psk_craft_state s, psk_craft_ep
     if (!state_ok(t, s) || ticks < 0 || (features_out && feat_ring <= 0)) return PSK_ERR_BADARG;
     if (s.n == 0 || ticks == 0) return PSK_OK;
     if (!expert_out || !ep.scen_grid || !ep.scen_idx || !ep.init_agent) return PSK_ERR_BADARG;
-    if (features_out && (reinterpret_cast<uintptr_t>(features_out) & 15)) return PSK_ERR_BADARG;
+    if (features_out && frame_misaligned(t, features_out, 16)) return PSK_ERR_BADARG;
     cudaStream_t st = (cudaStream_t)stream;
     int rc = PSK_ERR_UNSUPPORTED;
-    if (Medium::matches(t))
+    if (Medium::matches(t) && !generic_forced())
         rc = Medium::rollout(t, s, ep, ticks, action_in, features_out, feat_ring, expert_out, done_out,
                              success_out, stats, err_flags, st);
 

@@ -15,6 +15,7 @@
 #include <cuda_runtime.h>
 
 #include "../../include/psk_craft.h"
+#include "psk_common.cuh"
 #include "psk_hostcpu.h"
 
 #define PSK_HOST_STREAMS 3
@@ -406,7 +407,7 @@ int psk_craft_host_tick_resident(psk_craft_host_ctx *c, const uint8_t *host_acti
         return PSK_ERR_BADARG;
     if (!host_features) feature_format = PSK_FEATURES_NONE;
     DeviceScope scope(c->device);
-    if (n > 0 && n <= c->zerocopy_max && c->tables.width * c->tables.height <= 128) {
+    if (n > 0 && n <= c->zerocopy_max && psk::craft_fused_built(&c->tables)) {   // fused kernel only
         const int rc = tick_resident_zerocopy(c, host_action_in, host_features, feature_format, advance_first,
                                               host_expert, host_done, host_success, n, host_stats, host_err_flags);
         if (rc != PSK_ERR_UNSUPPORTED) return rc;

@@ -35,8 +35,11 @@ class VecCraft(object):
         self.tables = tables if tables is not None else CraftTables()
         self.ct = _lib.make_tables(self.tables)
         if not self.lib.psk_craft_supported(ctypes.byref(self.ct)):
-            raise _lib.PskError("world geometry %dx%d window %d is not built into libpsk_b200"
-                                % (self.tables.W, self.tables.H, self.tables.win_w))
+            raise _lib.PskError("world geometry %dx%d window %dx%d with %d kinds is outside what libpsk_b200 "
+                                "runs: 1 <= WIDTH, HEIGHT <= 64, odd WINDOW_WIDTH / WINDOW_HEIGHT from 1 to 9, "
+                                "at most 24 kinds"
+                                % (self.tables.W, self.tables.H, self.tables.win_w, self.tables.win_h,
+                                   self.tables.K))
         self.device = torch.device(device if device is not None else
                                    "cuda:%d" % torch.cuda.current_device())
         self.n = int(n)
